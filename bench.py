@@ -24,6 +24,7 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True      # the benchmark leaves the source tree as it found it (it may be read-only)
 
 METRIC = "train user-sequences/s (SASRec + BERT-base LoRA r=8 adapter-tuning step: fwd+bwd+allreduce+Adam)"
 UNIT = "user-seqs/s"
@@ -35,8 +36,13 @@ FLOP_FWD_PER_TOKEN = 12 * (14155776 + 92160 + 49152)   # SURVEY.md §8d: GEMMs +
 def parse():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=5)
+    ap.add_argument("--steps", type=int, default=5,
+                    help="timed training steps: of the headline loop and of the loops timed beside it (end to end, layouts, "
+                         "graphed step)")
     ap.add_argument("--warmup", type=int, default=3)
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last one computed to DIR/<name>.npy: loss (float64) and the "
+                         "trainable parameters after its Adam update and their gradients (float32, flat, trainer order)")
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--users", type=int, default=512, help="users per GPU per step (C2: 512)")
     ap.add_argument("--users-per-pass", type=int, default=512,
@@ -49,7 +55,10 @@ def parse():
     ap.add_argument("--no-variants", action="store_true", help="skip the extra (non-headline) unpadded-token measurement")
     ap.add_argument("--variants", default="all",
                     help="comma list of the non-headline variants to run: layouts (unpadded / dedup), graphed_step, c1, c3, c4")
-    return ap.parse_args()
+    a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    return a
 
 
 def make_args(r=8):
@@ -271,8 +280,8 @@ def reference_sd():
 
 
 def run_reference(a):
-    """--impl reference: the reference's CPU path (oracle port; the reference is Python and /root/reference does not
-    exist on the GPU box) on all host threads, each step a bounded sample of C2 (a.cpu_users users)."""
+    """--impl reference: the reference's CPU arithmetic (oracle port) on all host threads, each step a bounded sample of C2
+    (a.cpu_users users)."""
     import torch
     rank = int(os.environ.get("RANK", "0"))
     if rank != 0:
@@ -283,7 +292,7 @@ def run_reference(a):
     for _ in range(min(a.warmup, 1)):
         step()
     t0 = time.time()
-    steps = max(1, min(a.steps, 3))
+    steps = a.steps
     for _ in range(steps):
         step()
     dt = (time.time() - t0) / steps
@@ -468,6 +477,17 @@ def bench_item_table(model, args, catalogue, dev, world, rank):
 
 
 _REAL_STDOUT = None
+
+
+def dump_outputs(path, loss, trainer):
+    """What the last timed step computed, as a caller of trainer.train_step receives it: the loss it returns, and the
+    parameters and gradients it leaves in the trainer's flat buffers (317,696 fp32 values each for C2, parameter order of
+    trainer.names).  Inputs, initial weights and dropout seeds are fixed, so two builds can be compared array for array."""
+    import numpy as np
+    os.makedirs(path, exist_ok=True)
+    for name, t in (("loss", loss.detach().double().reshape(1)), ("params", trainer.flat_param),
+                    ("grads", trainer.flat_grad)):
+        np.save(os.path.join(path, name + ".npy"), t.cpu().numpy())
 
 
 def _time_steps(trainer, batches, steps, warmup, dev, world):
@@ -728,6 +748,8 @@ def main():
     ms = float(t)
     ms_per_step = ms / a.steps
     value = a.users * world / (ms_per_step / 1e3)
+    if a.dump_outputs and rank == 0:
+        dump_outputs(a.dump_outputs, loss, trainer)
 
     # ---------------- end-to-end: host (pinned) -> device copy of the batch + loss read-back every step ----------------
     barrier()

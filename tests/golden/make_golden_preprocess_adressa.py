@@ -2,7 +2,8 @@
 REAL tokenizer (transformers' BertTokenizer on the vocab.txt the reference ships under pretrained_models/bert/bert_base_uncased)
 on the REAL catalogue the reference ships (Dataset/Adressa/Adressa_news_base.tsv, 20,373 news titles, --num_words_title 30) and
 stores a digest of the token matrix in tests/golden/preprocess/adressa_digest.json.  This is the item side of BASELINE.json's
-configs[0] plumbing run.  The files stay in /root/reference; the test that uses this golden runs where they exist."""
+configs[0] plumbing run.  The files are not part of this repository, so the suite does not read the digest: it records what
+the unmodified readers produced (DESIGN.md cites its token count)."""
 import hashlib
 import importlib.util
 import json

@@ -1,7 +1,7 @@
 """Runs the UNMODIFIED image-tree readers (Downstream/CV/data_utils/preprocess.py: read_images, read_behaviors) on the REAL
 catalogue / behaviour files the reference ships (Dataset/Amazon/amazon_2w_{items,users}.tsv) and stores digests of what they
-return in tests/golden/preprocess/amazon_digest.json.  The data files stay in /root/reference; the test that uses this golden
-(tests/test_preprocess_cpu.py::test_image_tree_readers_on_the_reference_dataset) runs where they exist and is skipped elsewhere."""
+return in tests/golden/preprocess/amazon_digest.json.  The data files are not part of this repository, so the suite does not
+read the digest: it records what the unmodified readers returned on them."""
 import hashlib
 import importlib.util
 import json

@@ -118,36 +118,3 @@ def test_load_body_and_the_real_tokenizer(tmp_path):
     n = mask[1:].sum(1)
     assert (ids[1:, 0] == 2).all() and (ids[np.arange(1, len(ids)), n - 1] == 3).all()       # [CLS] ... [SEP]
     assert ((ids[1:] != 0) == (mask[1:] == 1)).all() and ids.max() < cfg.vocab_size and n.min() >= 2 and n.max() == L
-
-
-def test_image_tree_readers_on_the_reference_dataset():
-    """read_images + read_behaviors on the REAL files the reference ships (Dataset/Amazon: 14,720 items, 21,153 kept users)
-    against digests of what the unmodified Downstream/CV/data_utils/preprocess.py returned on them
-    (tests/golden/make_golden_preprocess_amazon.py).  The data stays in /root/reference: skipped where it is absent."""
-    import make_golden_preprocess_amazon as G
-    if not (os.path.exists(G.ITEMS) and os.path.exists(G.USERS)):
-        pytest.skip("the reference's dataset files are not on this machine")
-    from adapter4rec_b200.data_utils import preprocess as P
-    ref = json.load(open(os.path.join(F.DIR, "amazon_digest.json")))
-    keys, name_to_id = P.read_images(G.ITEMS)
-    assert len(name_to_id) == ref["before_items"] and keys[1] == next(iter(name_to_id)).encode("ascii")
-    out = P.read_behaviors(G.USERS, keys, name_to_id, ref["max_seq_len"], ref["min_seq_len"], logging.getLogger("preprocess_test"))
-    assert out[0] == ref["item_num"] and len(out[2]) == ref["users"]
-    assert G.digest(*out) == ref["sha256"]
-
-
-def test_text_readers_on_the_reference_catalogue_with_the_real_tokenizer():
-    """read_news_bert + get_doc_input_bert on the REAL Adressa catalogue the reference ships (20,373 titles) with transformers'
-    BertTokenizer on the reference's own vocab.txt: the [I+1, 60] token matrix equals, byte for byte, what the unmodified
-    readers produced (tests/golden/make_golden_preprocess_adressa.py) — the item side of BASELINE.json configs[0]'s plumbing
-    run.  Skipped where the reference's files are absent."""
-    import make_golden_preprocess_adressa as G
-    if not (os.path.exists(G.NEWS) and os.path.exists(G.BODY)):
-        pytest.skip("the reference's dataset / vocabulary files are not on this machine")
-    from transformers import BertTokenizer
-    from adapter4rec_b200.data_utils import preprocess as P
-    ref = json.load(open(os.path.join(F.DIR, "adressa_digest.json")))
-    content, name_to_id = G.token_matrix(P, BertTokenizer.from_pretrained(G.BODY))
-    assert content.shape == (ref["rows"], ref["cols"]) and len(name_to_id) == ref["names"]
-    assert abs(float(content[1:, 30:].sum(1).mean()) - ref["mean_tokens"]) < 1e-9
-    assert G.digest(content, name_to_id) == ref["sha256"]

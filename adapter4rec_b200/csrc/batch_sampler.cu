@@ -67,6 +67,7 @@ __global__ void __launch_bounds__(256) sample_gather_kernel(SampleParams p) {
       p.neg_out[slot] = neg;
       if (j < p.S1 - 1) p.log_mask[b * (p.S1 - 1) + j] = pos != 0 ? 1.0f : 0.0f;
     }
+    if (p.content == nullptr) continue;   // ids-only mode (the id item tower): the ids are seqs and neg_out themselves
     // gather: out[b, j, 0, :] = content[pos], out[b, j, 1, :] = content[neg]   (W int64 = W/2 uint4)
     const int vec = static_cast<int>(p.W >> 1);
     const uint4* src0 = reinterpret_cast<const uint4*>(p.content + pos * p.W);
@@ -84,11 +85,13 @@ __global__ void __launch_bounds__(256) sample_gather_kernel(SampleParams p) {
 extern "C" int a4r_sample_train_batch(const int64_t* seqs, const int64_t* item_content, const int64_t* neg_in, int64_t* out,
                                       float* log_mask, int64_t* neg_out, int32_t* fail_flag, int64_t B, int64_t S1,
                                       int64_t W, int64_t item_num, uint64_t seed, uint64_t offset, a4r_stream_t stream_) {
-  A4R_CHECK_ARG(B >= 0 && S1 >= 2 && W > 0 && W % 2 == 0 && item_num >= 1, "sample_train_batch: bad sizes (B=%lld S1=%lld W=%lld)",
-                (long long)B, (long long)S1, (long long)W);
+  const bool ids_only = item_content == nullptr;
+  A4R_CHECK_ARG(B >= 0 && S1 >= 2 && (ids_only ? W == 0 : (W > 0 && W % 2 == 0)) && item_num >= 1,
+                "sample_train_batch: bad sizes (B=%lld S1=%lld W=%lld)", (long long)B, (long long)S1, (long long)W);
   if (B == 0) return A4R_OK;   // empty batch: the (empty) output buffers may legitimately be NULL
-  A4R_CHECK_ARG(seqs && item_content && out && log_mask && neg_out && fail_flag, "sample_train_batch: NULL pointer");
-  A4R_CHECK_ARG(a4r_aligned16(item_content) && a4r_aligned16(out), "sample_train_batch: item_content / out must be 16B aligned");
+  A4R_CHECK_ARG(seqs && (ids_only || out) && log_mask && neg_out && fail_flag, "sample_train_batch: NULL pointer");
+  A4R_CHECK_ARG(ids_only || (a4r_aligned16(item_content) && a4r_aligned16(out)),
+                "sample_train_batch: item_content / out must be 16B aligned");
   int rc = a4r_device_check();
   if (rc != A4R_OK) return rc;
   SampleParams p;

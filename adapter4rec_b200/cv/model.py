@@ -4,7 +4,7 @@ import torch.nn as nn
 
 from .. import functional as Fn
 from ..model.encoders import User_Encoder
-from ..model.layers import BF16, to_2d_bf16
+from ..model.layers import BF16, IdEmbedding, to_2d_bf16
 from ..model.model import (CompacterModel, SASRecAdaptedSelfOutput, SASRecCompacterAdaptedSelfOutput,  # noqa: F401
                            SASRecParallelAdaptedSelfOutput, SASRecPfeifferVer2AdaptedSelfOutput,
                            check_trainable_supported)   # the SASRec wrappers are the text tree's classes (CV model.py:235-372,465-510)
@@ -48,26 +48,30 @@ class _ModelBase(nn.Module):
         self.user_encoder = User_Encoder(item_num=item_num, max_seq_len=args.max_seq_len, item_dim=args.embedding_dim,
                                          num_attention_heads=args.num_attention_heads, dropout=args.drop_rate,
                                          n_layers=args.transformer_block)
-        if not use_modal:
-            raise NotImplementedError("item_tower='id' is outside the modality-encoder hot path")
-        if 'vit' not in args.CV_model_load:
+        if not use_modal:                               # --item_tower id: the item table is a trainable embedding
+            self.id_embedding = IdEmbedding(item_num + 1, args.embedding_dim, padding_idx=0)
+        elif 'vit' not in args.CV_model_load:
             raise NotImplementedError("only the ViT image encoder is on the hot path (CV_model_load=%r)" % args.CV_model_load)
-        self.cv_encoder = Vit_Encoder(image_net=image_net)
+        else:
+            self.cv_encoder = Vit_Encoder(image_net=image_net)
         self.criterion = nn.BCEWithLogitsLoss()
         self._checked = None
 
     def forward(self, sample_items, log_mask, local_rank=None):
-        """sample_items f32 [B*(S+1)*2, 3, R, R]; log_mask f32 [B,S] -> scalar loss (Downstream/CV/model/model.py:54-77)."""
+        """sample_items f32 [B*(S+1)*2, 3, R, R] (the id tower: int64 item ids [B*(S+1)*2] or [B, S+1, 2]); log_mask f32
+        [B,S] -> scalar loss (Downstream/CV/model/model.py:54-77)."""
         if self.training:
             sig = tuple(p.requires_grad for p in self.parameters())
             if sig != self._checked:
                 check_trainable_supported(self)
                 self._checked = sig
-        input_embs_all = self.cv_encoder(sample_items)
-        D = self.args.embedding_dim
-        input_embs = input_embs_all.view(-1, self.max_seq_len + 1, 2, D)
-        input_logs_embs = input_embs[:, :-1, 0, :].contiguous()
-        log_mask = log_mask.to(device=input_embs_all.device, dtype=torch.float32).contiguous()
+        if not self.use_modal:
+            input_embs, input_logs_embs = self.id_embedding(sample_items.reshape(-1, self.max_seq_len + 1, 2))
+        else:
+            input_embs_all = self.cv_encoder(sample_items)
+            input_embs = input_embs_all.view(-1, self.max_seq_len + 1, 2, self.args.embedding_dim)
+            input_logs_embs = input_embs[:, :-1, 0, :].contiguous()
+        log_mask = log_mask.to(device=input_embs.device, dtype=torch.float32).contiguous()
         prec_vec = self.user_encoder(input_logs_embs, log_mask, local_rank)
         return Fn.bce_loss(prec_vec.contiguous(), input_embs.contiguous(), None if self.cpc else log_mask, cpc=self.cpc)
 

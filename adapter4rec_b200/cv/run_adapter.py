@@ -22,7 +22,7 @@ import torch.distributed as dist
 from torch.nn.init import constant_, xavier_normal_
 
 from .. import surgery
-from ..data_utils.metrics import eval_model, get_item_embeddings
+from ..data_utils.metrics import core_model, eval_model, get_item_embeddings
 from ..model.layers import Linear
 from ..run import _checkpoint_path, rank_shard, save_model, setup_seed  # noqa: F401  (same helpers as the text tree)
 from ..trainer import FlatAdamTrainer
@@ -46,9 +46,10 @@ def group_parameters_cv(model):
     return groups
 
 
-def build_model(args, item_num, local_rank, vit_config=None, vit_state_dict=None, model_dir=None):
-    """run_adapter.py:283-480 without the DDP wrap.  Only the ViT image tower is on this package's path ('vit' in
-    --CV_model_load); ResNet / MAE / CLIP towers are out of scope (DESIGN.md §7) and refused."""
+def build_vit(args, vit_config=None, vit_state_dict=None):
+    """run_adapter.py:283-297: the ViT-B/16 body with a fresh xavier `classifier` [768 -> embedding_dim].  Only the ViT image
+    tower is on this package's path ('vit' in --CV_model_load); ResNet / MAE / CLIP towers are out of scope (DESIGN.md §7)
+    and refused."""
     if 'vit' not in args.CV_model_load or 'mae' in args.CV_model_load:
         raise NotImplementedError("CV_model_load %r: only the ViT-B/16 tower is implemented" % args.CV_model_load)
     cv_model = ViTForImageClassification(vit_config if vit_config is not None else ViTConfigLite())
@@ -57,7 +58,14 @@ def build_model(args, item_num, local_rank, vit_config=None, vit_state_dict=None
     cv_model.classifier = Linear(cv_model.config.hidden_size, args.embedding_dim)        # :291-297
     xavier_normal_(cv_model.classifier.weight.data)
     constant_(cv_model.classifier.bias.data, 0)
-    model = (ModelCPC if "cpc" in args.arch else Model)(args, item_num, True, cv_model).to(local_rank)
+    return cv_model
+
+
+def build_model(args, item_num, local_rank, vit_config=None, vit_state_dict=None, model_dir=None, use_modal=True):
+    """run_adapter.py:283-480 without the DDP wrap.  use_modal = False (--item_tower id): no image body, the item table is
+    id_embedding (adapter insertion is refused: there is no body to insert into)."""
+    cv_model = build_vit(args, vit_config, vit_state_dict) if use_modal else None
+    model = (ModelCPC if "cpc" in args.arch else Model)(args, item_num, use_modal, cv_model).to(local_rank)
     if 'None' not in args.pretrained_recsys_model:                                     # :350-358
         ckpt = torch.load(_checkpoint_path("../pretrained_models/", args.pretrained_recsys_model), map_location="cpu",
                           weights_only=False)
@@ -77,11 +85,12 @@ def build_model(args, item_num, local_rank, vit_config=None, vit_state_dict=None
 class ImageBatches:
     """BuildTrainDataset / Build_Lmdb_Dataset.__getitem__ (Downstream/CV/data_utils/dataset.py:56-113) for a list of users:
     left-padded sequences, one uniform negative per position rejected against the user's own sequence, the images gathered
-    from the resident table: sample_items [B*(S+1)*2, 3, R, R] float32, log_mask [B, S]."""
+    from the resident table: sample_items [B*(S+1)*2, 3, R, R] float32, log_mask [B, S].  item_images None (the id tower):
+    sample_items are the item ids [B*(S+1)*2] int64 themselves."""
 
     def __init__(self, u2seq, item_images, item_num, max_seq_len, device, seed):
         self.u2seq, self.item_num, self.S, self.dev = u2seq, item_num, max_seq_len, device
-        self.images = torch.as_tensor(item_images, dtype=torch.float32).to(device)
+        self.images = None if item_images is None else torch.as_tensor(item_images, dtype=torch.float32).to(device)
         self.rng = random.Random(seed)
 
     def batch(self, users):
@@ -100,7 +109,7 @@ class ImageBatches:
                     neg = self.rng.randint(1, self.item_num)
                 ids[b, S1 - n + i, 1] = neg
         flat = torch.from_numpy(ids).view(-1).to(self.dev)
-        return self.images[flat], torch.from_numpy(log_mask).to(self.dev)
+        return flat if self.images is None else self.images[flat], torch.from_numpy(log_mask).to(self.dev)
 
 
 def synthetic_data(item_num=200, users=64, resize=224, max_seq_len=10, seed=0):
@@ -119,7 +128,7 @@ def synthetic_data(item_num=200, users=64, resize=224, max_seq_len=10, seed=0):
 
 def train(args, use_modal, local_rank, data, Log_file=None, vit_config=None, users_per_pass=32, model_dir=None):
     Log_file = Log_file or logging.getLogger("adapter4rec_b200.cv")
-    model = build_model(args, data.item_num, local_rank, vit_config)
+    model = build_model(args, data.item_num, local_rank, vit_config, use_modal=use_modal)
     start_epoch = 0
     trainer = FlatAdamTrainer(model, args.lr, args.fine_tune_lr, args.adapter_cv_lr, args.adapter_sasrec_lr,
                               users_per_pass=users_per_pass, grouping=group_parameters_cv)
@@ -138,7 +147,8 @@ def train(args, use_modal, local_rank, data, Log_file=None, vit_config=None, use
     world = dist.get_world_size() if dist.is_initialized() else 1
     users = sorted(data.users_train.keys())
     dev = next(model.parameters()).device
-    batches = ImageBatches(data.users_train, data.item_images, data.item_num, args.max_seq_len, dev, 12345 + rank)   # :681 seed
+    batches = ImageBatches(data.users_train, data.item_images if use_modal else None, data.item_num, args.max_seq_len, dev,
+                           12345 + rank)                                               # :681 seed
     max_hit10 = 0.0
     for ep in range(args.epoch):
         now_epoch = start_epoch + ep + 1
@@ -165,8 +175,10 @@ def train(args, use_modal, local_rank, data, Log_file=None, vit_config=None, use
 
 
 def run_eval(model, data, args, Log_file, v_or_t, local_rank, batch_size=256):
-    """run_adapter.py:632-660: the item table from the image tower, then full-ranking HR@10 / NDCG@10."""
-    table = get_item_embeddings(model, data.item_images, batch_size, args, True, local_rank)
+    """run_adapter.py:632-660: the item table from the image tower (or the id tower's embedding table), then full-ranking
+    HR@10 / NDCG@10."""
+    use_modal = core_model(model).use_modal
+    table = get_item_embeddings(model, data.item_images if use_modal else None, batch_size, args, use_modal, local_rank)
     hist, seqs = (data.users_history_for_valid, data.users_valid) if v_or_t == "valid" else \
         (data.users_history_for_test, data.users_test)
     return eval_model(model, hist, seqs, table, batch_size, args, data.item_num, Log_file, v_or_t, local_rank)

@@ -20,8 +20,9 @@ class BuildTrainDataset:
     contract for code that indexes it; `batch(users)` is the device path a training loop should call."""
 
     def __init__(self, u2seq, item_content, item_num, max_seq_len, use_modal=True, device=None, seed=123456):
-        if not use_modal:
-            raise NotImplementedError("item_tower='id' is outside the modality-encoder hot path")
+        """use_modal = False (the id item tower): item_content is not read (may be None) and a sample is the item ids
+        [S+1, 2] themselves; every id of u2seq must lie in [1, item_num] (checked here, once, on the host: the id tower's
+        table has exactly item_num + 1 rows)."""
         self.u2seq = u2seq
         self.item_num = item_num
         self.max_seq_len = max_seq_len + 1
@@ -29,8 +30,11 @@ class BuildTrainDataset:
         self.device = torch.device(device if device is not None else "cuda")
         self.seed = int(seed)
         self.batches_drawn = 0
-        content = torch.as_tensor(np.asarray(item_content) if not torch.is_tensor(item_content) else item_content)
-        self.item_content = content.to(device=self.device, dtype=torch.int64).contiguous()
+        if use_modal:
+            content = torch.as_tensor(np.asarray(item_content) if not torch.is_tensor(item_content) else item_content)
+            self.item_content = content.to(device=self.device, dtype=torch.int64).contiguous()
+        else:
+            self.item_content = None
         self.users = sorted(u2seq.keys())
         self._row = {u: i for i, u in enumerate(self.users)}
         S1 = self.max_seq_len
@@ -39,13 +43,18 @@ class BuildTrainDataset:
             s = list(u2seq[u])
             assert 2 <= len(s) <= S1, "sequence length must be in [2, max_seq_len + 1] (preprocess.py:51-59)"
             seqs[i, S1 - len(s):] = s                                  # left padding, dataset.py:34
+        if not use_modal and len(self.users):
+            real = seqs[seqs != 0]
+            if real.size != sum(len(u2seq[u]) for u in self.users) or real.min() < 1 or real.max() > item_num:
+                raise ValueError("item_tower id: every item id of the sequences must lie in [1, item_num = %d]" % item_num)
         self.seqs = torch.from_numpy(seqs).to(self.device)
 
     def __len__(self):
         return len(self.u2seq)
 
     def batch(self, users, neg_items=None, check=False):
-        """users: iterable of user ids -> (sample_items [B, S+1, 2, 2L] int64, log_mask [B, S] f32) on the device.
+        """users: iterable of user ids -> (sample_items [B, S+1, 2, 2L] int64, log_mask [B, S] f32) on the device; the
+        id tower's sample_items are the ids [B, S+1, 2] (history | negative).
         neg_items (optional int64 [B, S+1]) replays given negatives instead of sampling."""
         rows = torch.as_tensor([self._row[u] for u in users], dtype=torch.int64).to(self.device, non_blocking=True)
         seqs = self.seqs.index_select(0, rows)
@@ -56,6 +65,8 @@ class BuildTrainDataset:
         self.last_negatives = neg
         if check and int(fail.item()):
             raise RuntimeError("negative sampling found no admissible item (item_num <= max_seq_len + 1?)")
+        if out is None:
+            out = torch.stack([seqs, neg], -1)
         return out, log_mask
 
     def __getitem__(self, user_id):

@@ -80,10 +80,17 @@ def print_metrics(x, Log_file, v_or_t):
 
 def get_item_embeddings(model, item_content, test_batch_size, args, use_modal, local_rank):
     """metrics.py:62-79.  item_content [I+1, 2L] (numpy int or torch int64; row 0 = padding item).  Each rank encodes
-    ITS shard of item ids with the item encoder under no_grad and keeps it on the device (an ItemTable)."""
+    ITS shard of item ids with the item encoder under no_grad and keeps it on the device (an ItemTable).
+    use_modal = False (the id tower): the table is id_embedding.weight itself (item_content is not read); the rank's
+    shard is cast once to bf16 with the rounding of the training gather (RNE)."""
     module = core_model(model)
     module.eval()
     rank, world = _dist_info()
+    if not use_modal:
+        weight = module.id_embedding.weight.detach()
+        lo, hi = shard_range(weight.shape[0], rank, world)
+        emb, _ = ops.cast_transpose(weight[lo:hi], True, False) if hi > lo else (weight[:0].to(BF16), None)
+        return ItemTable(emb, lo, weight.shape[0], rank, world)
     rows = torch.as_tensor(np.asarray(item_content) if not torch.is_tensor(item_content) else item_content)
     image_tree = hasattr(module, "cv_encoder")       # Downstream/CV: item_content = images [I+1, 3, R, R] float32
     rows = rows.float() if image_tree else rows.long()

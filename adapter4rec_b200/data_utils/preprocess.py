@@ -116,16 +116,22 @@ def get_doc_input_bert(item_id_to_content, args):
     return news_title, news_title_attmask, None, None, None, None
 
 
-def load_text_data(args, tokenizer, Log_file):
+def load_text_data(args, tokenizer, Log_file, use_modal=True):
     """The reader block of run.py:319-341 in one call: the namespace `train(args, use_modal, local_rank, data)` of
     adapter4rec_b200.run / adapter4rec_b200.pretraining.text_run takes (item_content = the concatenation of the present
-    token / mask matrices, run.py:336-341)."""
+    token / mask matrices, run.py:336-341).  use_modal = False (the id tower): the catalogue is read by name only
+    (read_news, no tokenizer) and item_content is None."""
     import os
     root = os.path.join(args.root_data_dir, args.dataset)
-    before_dic, before_name_to_id = read_news_bert(os.path.join(root, args.news), args, tokenizer)
+    if use_modal:
+        before_dic, before_name_to_id = read_news_bert(os.path.join(root, args.news), args, tokenizer)
+    else:
+        before_dic, before_name_to_id = read_news(os.path.join(root, args.news))
     item_num, item_id_to_dic, users_train, users_valid, users_test, hist_valid, hist_test = read_behaviors(
         os.path.join(root, args.behaviors), before_dic, before_name_to_id, args.max_seq_len, args.min_seq_len, Log_file)
-    parts = [x for x in get_doc_input_bert(item_id_to_dic, args) if x is not None]
-    return types.SimpleNamespace(item_content=np.concatenate(parts, axis=1), item_num=item_num, users_train=users_train,
+    item_content = None
+    if use_modal:
+        item_content = np.concatenate([x for x in get_doc_input_bert(item_id_to_dic, args) if x is not None], axis=1)
+    return types.SimpleNamespace(item_content=item_content, item_num=item_num, users_train=users_train,
                                  users_valid=users_valid, users_test=users_test, users_history_for_valid=hist_valid,
                                  users_history_for_test=hist_test)

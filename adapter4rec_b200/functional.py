@@ -880,3 +880,41 @@ def houlsby_postln_block(x, inp, p, dense, intermediate, adapter, ln):
     return HoulsbyPostLNBlockFunction.apply(x, inp, p, w1, b1, c1, w2, b2, c2, adapter.fc_down.weight, adapter.fc_down.bias,
                                             adapter.fc_up.weight, adapter.fc_up.bias, ln.weight, ln.bias, ln.eps,
                                             adapter.act, adapter.fc_down._cache, adapter.fc_up._cache)
+
+
+class IdEmbeddingFunction(torch.autograd.Function):
+    """The id item tower's lookup (nn.Embedding(item_num + 1, D, padding_idx) reached from Model.forward with
+    use_modal = False): ids [B, S1, 2] -> (emb [B, S1, 2, D], hist [B, S1-1, D] = emb[:, :-1, 0]) bf16 from the fp32 master.
+
+    The backward adds the table gradient of BOTH outputs straight into `weight.grad` (created as zeros when absent) and
+    returns None for the weight: the trainer's `.grad` is a view into its flat buffer, and a returned dense [V, D] tensor
+    would make autograd allocate, zero, add and free a full-table temporary per pass for a gradient that touches at most
+    B*S1*2 rows.  Rows are summed in fp32 in a fixed order without atomics (bit-identical run to run and under a graph
+    replay); row padding_idx is never written."""
+
+    @staticmethod
+    def forward(ctx, ids, weight, padding_idx):
+        emb, hist = ops.id_embed_fwd(weight.detach(), ids)
+        ctx.save_for_backward(ids)
+        ctx.weight, ctx.padding_idx = weight, padding_idx
+        return emb, hist
+
+    @staticmethod
+    def backward(ctx, d_emb, d_hist):
+        (ids,) = ctx.saved_tensors
+        w = ctx.weight
+        if d_emb is None and d_hist is None:
+            return None, None, None
+        if w.grad is None:
+            w.grad = torch.zeros_like(w)
+        ref = d_emb if d_emb is not None else d_hist
+        B, S1 = ids.shape[0], ids.shape[1]
+        if d_emb is None:
+            d_emb = torch.zeros((B, S1, 2, w.shape[1]), dtype=ref.dtype, device=ref.device)
+        ops.id_embed_bwd(ids, d_emb.contiguous(), None if d_hist is None else d_hist.contiguous(), w.grad,
+                         padding_idx=ctx.padding_idx, accumulate=True)
+        return None, None, None
+
+
+def id_embedding(ids, weight, padding_idx=0):
+    return IdEmbeddingFunction.apply(ids, weight, padding_idx)

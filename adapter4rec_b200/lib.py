@@ -126,6 +126,9 @@ PROTOTYPES = {
     "a4r_gather_rows": (c_int32, [c_void_p, c_void_p, c_void_p, c_int64, c_int64, c_void_p]),
     "a4r_sample_train_batch": (c_int32, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int64,
                                          c_int64, c_int64, c_int64, ctypes.c_uint64, ctypes.c_uint64, c_void_p]),
+    "a4r_id_embed_fwd": (c_int32, [c_void_p, c_int64, c_int64, c_void_p, c_int64, c_int64, c_void_p, c_void_p, c_void_p]),
+    "a4r_id_embed_bwd": (c_int32, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int64, c_int64, c_int64, c_int64,
+                                   c_int64, c_int32, c_void_p]),
     "a4r_score_topk_partials": (c_int32, [c_int64, c_int64]),
     "a4r_score_topk": (c_int32, [c_void_p, c_int64, c_void_p, c_int64, c_int64, c_int64, c_int64, c_int64, c_void_p,
                                  c_int64, c_int32, c_void_p, c_void_p, c_void_p]),

@@ -142,3 +142,25 @@ class Embedding(nn.Module):
 
     def table_bf16(self):
         return self._cache.get(self.weight)[0]
+
+
+class IdEmbedding(nn.Module):
+    """The id item tower's table: nn.Embedding(num_embeddings, embedding_dim, padding_idx=0) with the parameter name
+    `weight` [V, D] (fp32 master, xavier_normal_ as the reference initialises id_embedding; row padding_idx is zero and is
+    never written by the backward).  forward(ids [B, S1, 2] int64) -> (emb bf16 [B, S1, 2, D], hist bf16 [B, S1-1, D]):
+    the lookup and the user-encoder input in one kernel (Fn.IdEmbeddingFunction)."""
+
+    def __init__(self, num_embeddings, embedding_dim, padding_idx=0):
+        super().__init__()
+        self.num_embeddings, self.embedding_dim, self.padding_idx = num_embeddings, embedding_dim, padding_idx
+        self.weight = nn.Parameter(torch.empty(num_embeddings, embedding_dim))
+        nn.init.xavier_normal_(self.weight)
+        with torch.no_grad():
+            self.weight[padding_idx].zero_()
+
+    def forward(self, ids):
+        ids = ids.to(device=self.weight.device, dtype=torch.int64).contiguous()
+        return Fn.id_embedding(ids, self.weight, self.padding_idx)
+
+    def extra_repr(self):
+        return "%d, %d, padding_idx=%d" % (self.num_embeddings, self.embedding_dim, self.padding_idx)

@@ -7,7 +7,7 @@ import torch.nn as nn
 from .. import functional as Fn
 from .. import ops
 from .encoders import Bert_Encoder, User_Encoder
-from .layers import BF16, Embedding, to_2d_bf16
+from .layers import BF16, Embedding, IdEmbedding, to_2d_bf16
 from .layers import LayerNorm
 from .layers import PHMLinear
 from .layers import Linear
@@ -45,8 +45,8 @@ class _ModelBase(nn.Module):
         self.l2_weight = args.l2_weight / 2
         if self.use_modal:
             self.bert_encoder = Bert_Encoder(args=args, bert_model=bert_model)
-        else:
-            raise NotImplementedError("item_tower='id' (nn.Embedding item table) is outside the modality-encoder hot path")
+        else:                                           # --item_tower id: the item table is a trainable embedding
+            self.id_embedding = IdEmbedding(item_num + 1, args.embedding_dim, padding_idx=0)
         self.user_encoder = User_Encoder(item_num=item_num, max_seq_len=args.max_seq_len, item_dim=args.embedding_dim,
                                          num_attention_heads=args.num_attention_heads, dropout=args.drop_rate,
                                          n_layers=args.transformer_block)
@@ -54,7 +54,8 @@ class _ModelBase(nn.Module):
         self._checked = None
 
     def forward(self, sample_items, log_mask, local_rank=None, sample_items_id=None, cand_bias=None):
-        """sample_items int64 [B*(S+1)*2, 2L] (ids | mask rows), log_mask f32 [B,S] -> scalar loss.
+        """sample_items int64 [B*(S+1)*2, 2L] (ids | mask rows), log_mask f32 [B,S] -> scalar loss.  The id tower
+        (use_modal = False) takes the item ids themselves: int64 [B*(S+1)*2] or [B, S+1, 2].
 
         Extension beyond the reference signature (model.py:48): with `args.loss_type == "inbatch_softmax"` (an attribute,
         not a command-line flag — the flag set stays the reference's) the BCE head is replaced by the in-batch softmax
@@ -65,7 +66,10 @@ class _ModelBase(nn.Module):
             if sig != self._checked:
                 check_trainable_supported(self)
                 self._checked = sig
-        if getattr(self, "dedup_items", False):
+        D = self.args.embedding_dim
+        if not self.use_modal:
+            input_embs, input_logs_embs = self.id_embedding(sample_items.reshape(-1, self.max_seq_len, 2))
+        elif getattr(self, "dedup_items", False):
             # Optional (off by default, not what the reference executes): an item that occurs several times in the batch
             # — as a positive of several users, as a sampled negative, as the padding row — is encoded ONCE and its
             # embedding row is shared; the backward sums the gradient rows of its occurrences.  Identical forward values
@@ -75,15 +79,15 @@ class _ModelBase(nn.Module):
             input_embs_all = Fn.expand_rows(self.bert_encoder(uniq), inverse, counts)
         else:
             input_embs_all = self.bert_encoder(sample_items)                   # [N, D] bf16
-        D = self.args.embedding_dim
-        input_embs = input_embs_all.view(-1, self.max_seq_len, 2, D)
-        input_logs_embs = input_embs[:, :-1, 0, :].contiguous()                # history items 0..S-1 as user-encoder input
-        log_mask = log_mask.to(device=input_embs_all.device, dtype=torch.float32).contiguous()
+        if self.use_modal:
+            input_embs = input_embs_all.view(-1, self.max_seq_len, 2, D)
+            input_logs_embs = input_embs[:, :-1, 0, :].contiguous()            # history items 0..S-1 as user-encoder input
+        log_mask = log_mask.to(device=input_embs.device, dtype=torch.float32).contiguous()
         prec_vec = self.user_encoder(input_logs_embs, log_mask, local_rank)
         if getattr(self.args, "loss_type", "bce") == "inbatch_softmax":
             if self.cpc or sample_items_id is None:
                 raise ValueError("loss_type='inbatch_softmax' needs sample_items_id [B, S+1] and is not defined for ModelCPC")
-            ids = sample_items_id.to(device=input_embs_all.device, dtype=torch.int64).view(-1, self.max_seq_len).contiguous()
+            ids = sample_items_id.to(device=input_embs.device, dtype=torch.int64).view(-1, self.max_seq_len).contiguous()
             return Fn.inbatch_softmax_loss(prec_vec.contiguous(), input_embs.contiguous(), ids, log_mask, cand_bias)
         return Fn.bce_loss(prec_vec.contiguous(), input_embs.contiguous(), None if self.cpc else log_mask, cpc=self.cpc)
 

@@ -535,13 +535,17 @@ def gather_rows(table, ids):
 
 def sample_train_batch(seqs, item_content, item_num, seed, offset, neg_in=None):
     """seqs int64 [B, S1] (left-padded ids), item_content int64 [I+1, W] -> (sample_items [B, S1, 2, W] int64,
-    log_mask [B, S1-1] f32, neg ids [B, S1] int64, fail flag [1] int32 — left on the device, no sync here)."""
+    log_mask [B, S1-1] f32, neg ids [B, S1] int64, fail flag [1] int32 — left on the device, no sync here).
+    item_content None: ids-only mode, sample_items is None (the id tower's sample is stack([seqs, neg], -1))."""
     assert seqs.dtype == torch.int64 and seqs.is_contiguous() and seqs.dim() == 2
-    assert item_content.dtype == torch.int64 and item_content.is_contiguous() and item_content.dim() == 2
     B, S1 = seqs.shape
-    W = item_content.shape[1]
     dev = seqs.device
-    out = torch.empty((B, S1, 2, W), dtype=torch.int64, device=dev)
+    if item_content is None:
+        W, out = 0, None
+    else:
+        assert item_content.dtype == torch.int64 and item_content.is_contiguous() and item_content.dim() == 2
+        W = item_content.shape[1]
+        out = torch.empty((B, S1, 2, W), dtype=torch.int64, device=dev)
     log_mask = torch.empty((B, S1 - 1), dtype=torch.float32, device=dev)
     neg = torch.empty((B, S1), dtype=torch.int64, device=dev)
     fail = torch.zeros(1, dtype=torch.int32, device=dev)
@@ -551,6 +555,36 @@ def sample_train_batch(seqs, item_content, item_num, seed, offset, neg_in=None):
                                                  _p(fail), B, S1, W, int(item_num), int(seed) & (2 ** 64 - 1),
                                                  int(offset) & (2 ** 64 - 1), _stream()), "a4r_sample_train_batch")
     return out, log_mask, neg, fail
+
+
+def id_embed_fwd(table, ids, want_hist=True):
+    """table f32 [V, D] (the fp32 master), ids int64 [B, S1, 2] -> (emb bf16 [B, S1, 2, D], hist bf16 [B, S1-1, D] or
+    None): bf16_rne(table[ids]) and its history slots, in one pass."""
+    assert table.dtype == torch.float32 and table.dim() == 2 and table.is_contiguous()
+    assert ids.dtype == torch.int64 and ids.dim() == 3 and ids.shape[2] == 2 and ids.is_contiguous()
+    B, S1, _ = ids.shape
+    V, D = table.shape
+    emb = torch.empty((B, S1, 2, D), dtype=BF16, device=table.device)
+    hist = torch.empty((B, S1 - 1, D), dtype=BF16, device=table.device) if want_hist else None
+    _l.check(_l.get_lib().a4r_id_embed_fwd(_p(table), V, D, _p(ids), B, S1, _p(emb), _p(hist), _stream()),
+             "a4r_id_embed_fwd")
+    return emb, hist
+
+
+def id_embed_bwd(ids, d_emb, d_hist, grad, padding_idx=0, accumulate=True):
+    """grad f32 [V, D] (+)= the table gradient of id_embed_fwd's two outputs (d_hist may be None), summed per row in fp32 in
+    ascending occurrence order.  The occurrences are grouped by a stable device sort of the ids (no host sync)."""
+    assert ids.dtype == torch.int64 and ids.dim() == 3 and ids.shape[2] == 2 and ids.is_contiguous()
+    B, S1, _ = ids.shape
+    V, D = grad.shape
+    assert grad.dtype == torch.float32 and grad.is_contiguous()
+    assert d_emb.dtype == BF16 and d_emb.is_contiguous() and d_emb.numel() == B * S1 * 2 * D
+    if d_hist is not None:
+        assert d_hist.dtype == BF16 and d_hist.is_contiguous() and d_hist.numel() == B * (S1 - 1) * D
+    sorted_ids, order = torch.sort(ids.view(-1), stable=True)
+    _l.check(_l.get_lib().a4r_id_embed_bwd(_p(sorted_ids), _p(order), _p(d_emb), _p(d_hist), _p(grad), V, D, B, S1,
+                                           int(padding_idx), int(bool(accumulate)), _stream()), "a4r_id_embed_bwd")
+    return grad
 
 
 def score_topk(users, items, id_base=0, history=None, k=10):

@@ -8,40 +8,33 @@ validation users (batch 256) and writes epoch-{n}.pt (:258-268).
 
 No adapters: every unfrozen tensor of the ViT trains (patch projection, cls token, position embeddings included; DESIGN.md
 §4.4).  Precision: the reference's fp16 autocast + GradScaler (:229,245-250) has no counterpart — bf16 compute with fp32
-accumulation and fp32 master weights needs no loss scaling.  ResNet / MAE towers and the id tower are out of scope (DESIGN.md
-§7).  The LMDB reader is host-side: the caller hands in the arrays it produces, as for adapter4rec_b200.cv.run_adapter."""
+accumulation and fp32 master weights needs no loss scaling.  ResNet / MAE towers are out of scope (DESIGN.md §7); --item_tower
+id (use_modal = False) trains the ID-embedding table and the user encoder.  The LMDB reader is host-side: the caller hands in the arrays it produces, as for adapter4rec_b200.cv.run_adapter."""
 import logging
 import random
 import re
 
 import torch
 import torch.distributed as dist
-from torch.nn.init import constant_, xavier_normal_
 
 from ..cv.model import Model, ModelCPC
-from ..cv.run_adapter import ImageBatches, group_parameters_cv, run_eval, synthetic_data  # noqa: F401
-from ..cv.vit import ViTConfigLite, ViTForImageClassification
-from ..model.layers import Linear
+from ..cv.run_adapter import ImageBatches, build_vit, group_parameters_cv, run_eval, synthetic_data  # noqa: F401
 from ..run import _checkpoint_path, rank_shard, save_model, setup_seed  # noqa: F401
 from ..trainer import FlatAdamTrainer
 
 
-def build_model(args, item_num, local_rank, vit_config=None, vit_state_dict=None, downstream=False):
+def build_model(args, item_num, local_rank, vit_config=None, vit_state_dict=None, downstream=False, use_modal=True):
     """Pretraining/CV/run.py:91-147 (downstream=False) / Downstream/CV/run.py:98-164 (downstream=True: always Model, and
-    --pretrained_recsys_model is loaded right after construction) without the DDP wrap."""
-    if 'vit' not in args.CV_model_load or 'mae' in args.CV_model_load:
-        raise NotImplementedError("CV_model_load %r: only the ViT-B/16 tower is implemented" % args.CV_model_load)
-    cv_model = ViTForImageClassification(vit_config if vit_config is not None else ViTConfigLite())
-    if vit_state_dict is not None:
-        cv_model.load_state_dict(vit_state_dict, strict=False)
-    cv_model.classifier = Linear(cv_model.config.hidden_size, args.embedding_dim)
-    xavier_normal_(cv_model.classifier.weight.data)
-    constant_(cv_model.classifier.bias.data, 0)
-    for index, (_, param) in enumerate(cv_model.named_parameters()):
-        if index < args.freeze_paras_before:
-            param.requires_grad = False
+    --pretrained_recsys_model is loaded right after construction) without the DDP wrap.  use_modal = False (--item_tower
+    id): no image body, the item table is id_embedding."""
+    cv_model = None
+    if use_modal:
+        cv_model = build_vit(args, vit_config, vit_state_dict)
+        for index, (_, param) in enumerate(cv_model.named_parameters()):
+            if index < args.freeze_paras_before:
+                param.requires_grad = False
     cls = Model if downstream or "sasrec" in args.arch else ModelCPC
-    model = cls(args, item_num, True, cv_model).to(local_rank)
+    model = cls(args, item_num, use_modal, cv_model).to(local_rank)
     if downstream and 'None' not in args.pretrained_recsys_model:
         ckpt = torch.load(_checkpoint_path("../pretrained_models/", args.pretrained_recsys_model), map_location="cpu",
                           weights_only=False)
@@ -51,10 +44,8 @@ def build_model(args, item_num, local_rank, vit_config=None, vit_state_dict=None
 
 def train(args, use_modal, local_rank, data, Log_file=None, vit_config=None, users_per_pass=32, model_dir=None,
           downstream=False):
-    if not use_modal:
-        raise NotImplementedError("item_tower='id' is outside the modality-encoder hot path")
     Log_file = Log_file or logging.getLogger("adapter4rec_b200.pretraining.cv")
-    model = build_model(args, data.item_num, local_rank, vit_config, downstream=downstream)
+    model = build_model(args, data.item_num, local_rank, vit_config, downstream=downstream, use_modal=use_modal)
     trainer = FlatAdamTrainer(model, args.lr, args.fine_tune_lr, args.fine_tune_lr, args.lr, users_per_pass=users_per_pass,
                               grouping=group_parameters_cv)
     Log_file.info("##### trainable_num {} #####".format(trainer.num_trainable))
@@ -73,7 +64,8 @@ def train(args, use_modal, local_rank, data, Log_file=None, vit_config=None, use
     world = dist.get_world_size() if dist.is_initialized() else 1
     users = sorted(data.users_train.keys())
     dev = next(model.parameters()).device
-    batches = ImageBatches(data.users_train, data.item_images, data.item_num, args.max_seq_len, dev, 12345 + rank)
+    batches = ImageBatches(data.users_train, data.item_images if use_modal else None, data.item_num, args.max_seq_len, dev,
+                           12345 + rank)
     max_hit10, max_epoch = 0.0, 0
     for ep in range(args.epoch):
         now_epoch = start_epoch + ep + 1
@@ -102,7 +94,7 @@ def train(args, use_modal, local_rank, data, Log_file=None, vit_config=None, use
 def test(args, use_modal, local_rank, data, Log_file=None, vit_config=None, model_dir=None, downstream=False):
     """Pretraining/CV/run.py:25-77: build, load --load_ckpt_name if given, rank the TEST users."""
     Log_file = Log_file or logging.getLogger("adapter4rec_b200.pretraining.cv")
-    model = build_model(args, data.item_num, local_rank, vit_config, downstream=downstream)
+    model = build_model(args, data.item_num, local_rank, vit_config, downstream=downstream, use_modal=use_modal)
     if 'None' not in args.load_ckpt_name:
         ckpt = torch.load(_checkpoint_path(model_dir, args.load_ckpt_name), map_location="cpu", weights_only=False)
         model.load_state_dict(ckpt['model_state_dict'])

@@ -8,7 +8,8 @@ downstream script loads through --pretrained_model_name.
 There are no adapters here: every unfrozen tensor of the body trains, so the backward is the full fine-tuning path (weight
 gradients on the tcgen05 split-token kernel, embedding-table scatter-adds; DESIGN.md §4.4).  Precision: the reference wraps the
 step in fp16 autocast + GradScaler (run.py:301,319-324); this package computes in bf16 with fp32 accumulation and fp32 master
-weights, which needs no loss scaling.  The OPT bodies of run.py:135-140 and the id tower are out of scope (DESIGN.md §7).
+weights, which needs no loss scaling.  The OPT bodies of run.py:135-140 are out of scope (DESIGN.md §7).  --item_tower id
+trains the ID-embedding table (id_embedding.weight, in the --lr group) and the user encoder; no body is read.
 The TSV readers / tokeniser are host-side: the caller hands in the arrays they produce, as for adapter4rec_b200.run."""
 import logging
 import random
@@ -50,8 +51,10 @@ def group_parameters_pretrain(model):
     return groups
 
 
-def build_model(args, item_num, local_rank, bert_config=None, bert_state_dict=None):
-    """run.py:127-218 without the DDP wrap."""
+def build_model(args, item_num, local_rank, bert_config=None, bert_state_dict=None, use_modal=True):
+    """run.py:127-218 without the DDP wrap; use_modal = False (--item_tower id): no body, the item table is id_embedding."""
+    if not use_modal:
+        return (Model if 'sasrec' in args.arch else ModelCPC)(args, item_num, False, None).to(local_rank)
     if 'opt' in args.bert_model_load:
         raise NotImplementedError("bert_model_load %r: the OPT bodies are outside the hot path" % args.bert_model_load)
     cfg = bert_config if bert_config is not None else TextConfigLite()
@@ -67,10 +70,8 @@ def build_model(args, item_num, local_rank, bert_config=None, bert_state_dict=No
 
 def train(args, use_modal, local_rank, data, Log_file=None, bert_config=None, users_per_pass=128, model_dir=None,
           bert_state_dict=None):
-    if not use_modal:
-        raise NotImplementedError("item_tower='id' is outside the modality-encoder hot path")
     Log_file = Log_file or logging.getLogger("adapter4rec_b200.pretraining")
-    model = build_model(args, data.item_num, local_rank, bert_config, bert_state_dict)
+    model = build_model(args, data.item_num, local_rank, bert_config, bert_state_dict, use_modal)
     trainer = FlatAdamTrainer(model, args.lr, args.fine_tune_lr, args.lr, args.lr, users_per_pass=users_per_pass,
                               grouping=group_parameters_pretrain)
     Log_file.info("##### trainable_num {} #####".format(trainer.num_trainable))
@@ -88,7 +89,7 @@ def train(args, use_modal, local_rank, data, Log_file=None, bert_config=None, us
         if ckpt.get('cuda_rng_state') is not None and torch.cuda.is_available():
             torch.cuda.set_rng_state(ckpt['cuda_rng_state'])
     users = sorted(data.users_train.keys())
-    train_ds = BuildTrainDataset(data.users_train, data.item_content, data.item_num, args.max_seq_len, True,
+    train_ds = BuildTrainDataset(data.users_train, data.item_content, data.item_num, args.max_seq_len, use_modal,
                                  device=next(model.parameters()).device, seed=123456 + rank)    # run.py:398 seed
     max_hit10, max_epoch = 0.0, 0
     for ep in range(args.epoch):
@@ -116,7 +117,7 @@ def train(args, use_modal, local_rank, data, Log_file=None, bert_config=None, us
 def test(args, use_modal, local_rank, data, Log_file=None, bert_config=None, model_dir=None, bert_state_dict=None):
     """run.py:32-118: build, load --load_ckpt_name, rank the TEST users."""
     Log_file = Log_file or logging.getLogger("adapter4rec_b200.pretraining")
-    model = build_model(args, data.item_num, local_rank, bert_config, bert_state_dict)
+    model = build_model(args, data.item_num, local_rank, bert_config, bert_state_dict, use_modal)
     if 'None' not in args.load_ckpt_name:
         ckpt = torch.load(_checkpoint_path(model_dir, args.load_ckpt_name), map_location="cpu", weights_only=False)
         model.load_state_dict(ckpt['model_state_dict'])
@@ -131,8 +132,7 @@ def main(argv=None, pretrained_root="../pretrained_models", users_per_pass=128):
     from ..run import _file_logger, load_body
     from .text_parameters import parse_args
     args = parse_args(argv)
-    if 'modal' not in args.item_tower:
-        raise NotImplementedError("item_tower='id' is outside the modality-encoder hot path")
+    use_modal = 'modal' in args.item_tower                              # run.py:405-408
     local_rank = int(os.environ.get("LOCAL_RANK", max(args.local_rank, 0)))
     torch.cuda.set_device(local_rank)
     if "RANK" in os.environ and not dist.is_initialized():
@@ -147,12 +147,12 @@ def main(argv=None, pretrained_root="../pretrained_models", users_per_pass=128):
     Log_file = _file_logger("Log_file", './logs_' + dir_label + ('_test' if 'test' in args.mode else '_train'), rank)
     Log_file.info(args)
     os.makedirs(model_dir, exist_ok=True)
-    tokenizer, cfg, state = load_body(args, pretrained_root)
-    data = load_text_data(args, tokenizer, Log_file)
+    tokenizer, cfg, state = load_body(args, pretrained_root) if use_modal else (None, None, None)
+    data = load_text_data(args, tokenizer, Log_file, use_modal)
     if 'train' in args.mode:
-        return train(args, True, local_rank, data, Log_file, cfg, users_per_pass, model_dir, bert_state_dict=state)
+        return train(args, use_modal, local_rank, data, Log_file, cfg, users_per_pass, model_dir, bert_state_dict=state)
     if 'test' in args.mode:
-        return test(args, True, local_rank, data, Log_file, cfg, model_dir, bert_state_dict=state)
+        return test(args, use_modal, local_rank, data, Log_file, cfg, model_dir, bert_state_dict=state)
 
 
 if __name__ == "__main__":

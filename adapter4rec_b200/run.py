@@ -19,7 +19,7 @@ import torch.distributed as dist
 from . import functional as Fn
 from . import surgery
 from .data_utils.dataset import BuildTrainDataset
-from .data_utils.metrics import eval_model, get_item_embeddings
+from .data_utils.metrics import core_model, eval_model, get_item_embeddings
 from .model import BertModel, Model, ModelCPC, RobertaModel, TextConfigLite
 from .trainer import FlatAdamTrainer
 
@@ -98,20 +98,23 @@ def _checkpoint_path(directory, name):
     return path
 
 
-def build_model(args, item_num, local_rank, bert_config=None, bert_state_dict=None):
+def build_model(args, item_num, local_rank, bert_config=None, bert_state_dict=None, use_modal=True):
     """run.py:286-503 without the DDP wrap (the trainer owns the gradient all-reduce): body -> prefix/pooler freeze ->
     Model / ModelCPC -> fine_tune_to freeze -> --pretrained_model_name checkpoint (BEFORE the surgery, run.py:374-381) ->
-    adapter insertion -> LayerNorm unfreeze."""
-    cfg = bert_config if bert_config is not None else TextConfigLite()
-    roberta = 'roberta' in args.bert_model_load
-    bert_model = (RobertaModel if roberta else BertModel)(cfg)
-    if bert_state_dict is not None:
-        bert_model.load_state_dict(bert_state_dict, strict=False)
-    freeze_bert_prefix(bert_model, args)
-    if args.word_embedding_dim != cfg.hidden_size:
-        raise ValueError("bert_model_load %r implies hidden width %d, the body has %d"
-                         % (args.bert_model_load, args.word_embedding_dim, cfg.hidden_size))
-    model = (ModelCPC if "cpc" in args.arch else Model)(args, item_num, True, bert_model).to(local_rank)
+    adapter insertion -> LayerNorm unfreeze.  use_modal = False (--item_tower id): no body; the model's item table is
+    id_embedding and there is nothing to insert adapters into (surgery refuses)."""
+    bert_model = None
+    if use_modal:
+        cfg = bert_config if bert_config is not None else TextConfigLite()
+        roberta = 'roberta' in args.bert_model_load
+        bert_model = (RobertaModel if roberta else BertModel)(cfg)
+        if bert_state_dict is not None:
+            bert_model.load_state_dict(bert_state_dict, strict=False)
+        freeze_bert_prefix(bert_model, args)
+        if args.word_embedding_dim != cfg.hidden_size:
+            raise ValueError("bert_model_load %r implies hidden width %d, the body has %d"
+                             % (args.bert_model_load, args.word_embedding_dim, cfg.hidden_size))
+    model = (ModelCPC if "cpc" in args.arch else Model)(args, item_num, use_modal, bert_model).to(local_rank)
     if 'None' in args.fine_tune_to:
         surgery.freeze_all(model)
     elif 'all' not in args.fine_tune_to:
@@ -153,7 +156,7 @@ def train(args, use_modal, local_rank, data, Log_file=None, bert_config=None, us
     """graphed=True replays each step from a CUDA graph per rank (trainer.train_step_graphed: bit-identical arithmetic, one
     recording per batch shape); the default is the eager step."""
     Log_file = Log_file or logging.getLogger("adapter4rec_b200")
-    model = build_model(args, data.item_num, local_rank, bert_config, bert_state_dict)
+    model = build_model(args, data.item_num, local_rank, bert_config, bert_state_dict, use_modal)
     trainer = FlatAdamTrainer(model, args.lr, args.fine_tune_lr, args.adapter_bert_lr, args.adapter_sasrec_lr,
                               users_per_pass=users_per_pass)
     Log_file.info("##### trainable_num {} #####".format(trainer.num_trainable))
@@ -171,7 +174,7 @@ def train(args, use_modal, local_rank, data, Log_file=None, bert_config=None, us
         if ckpt.get('cuda_rng_state') is not None and torch.cuda.is_available():
             torch.cuda.set_rng_state(ckpt['cuda_rng_state'])
     users = sorted(data.users_train.keys())
-    train_ds = BuildTrainDataset(data.users_train, data.item_content, data.item_num, args.max_seq_len, True,
+    train_ds = BuildTrainDataset(data.users_train, data.item_content, data.item_num, args.max_seq_len, use_modal,
                                  device=next(model.parameters()).device, seed=123456 + rank)   # run.py:686 seed; per-rank stream
     max_hit10, max_eval, max_epoch, now_epoch = 0.0, 0.0, 0, start_epoch
     # utils.py:90-102 (para_and_log): --logging_num progress lines per epoch
@@ -212,8 +215,9 @@ def train(args, use_modal, local_rank, data, Log_file=None, bert_config=None, us
 
 
 def run_eval(model, data, args, Log_file, v_or_t, local_rank, batch_size=512):
-    """run.py:649-670: item table, then full-ranking HR@10 / NDCG@10."""
-    table = get_item_embeddings(model, data.item_content, batch_size, args, True, local_rank)
+    """run.py:649-670: item table (the item encoder's, or the id tower's embedding table), then full-ranking HR@10 /
+    NDCG@10."""
+    table = get_item_embeddings(model, data.item_content, batch_size, args, core_model(model).use_modal, local_rank)
     hist, seqs = (data.users_history_for_valid, data.users_valid) if v_or_t == "valid" else \
         (data.users_history_for_test, data.users_test)
     return eval_model(model, hist, seqs, table, batch_size, args, data.item_num, Log_file, v_or_t, local_rank)
@@ -223,7 +227,7 @@ def test(args, use_modal, local_rank, data, Log_file=None, bert_config=None, ber
     """run.py:86-275 (--mode test): the model built as for training, --load_ckpt_name from model_dir (a missing file is an
     error), then the TEST users ranked."""
     Log_file = Log_file or logging.getLogger("adapter4rec_b200")
-    model = build_model(args, data.item_num, local_rank, bert_config, bert_state_dict)
+    model = build_model(args, data.item_num, local_rank, bert_config, bert_state_dict, use_modal)
     if 'None' not in args.load_ckpt_name:
         ckpt = torch.load(_checkpoint_path(model_dir, args.load_ckpt_name), map_location="cpu", weights_only=False)
         model.load_state_dict(ckpt['model_state_dict'])
@@ -284,12 +288,13 @@ def main(argv=None, pretrained_root="../pretrained_models", users_per_pass=128):
     Log_file = _file_logger("Log_file", './logs_' + dir_label + ('_test' if 'test' in args.mode else '_train'), rank)
     Log_file.info(args)
     os.makedirs(model_dir, exist_ok=True)
-    tokenizer, cfg, state = load_body(args, pretrained_root)
-    data = load_text_data(args, tokenizer, Log_file)
+    use_modal = 'modal' in args.item_tower                      # run.py:695-698
+    tokenizer, cfg, state = load_body(args, pretrained_root) if use_modal else (None, None, None)
+    data = load_text_data(args, tokenizer, Log_file, use_modal)
     if 'train' in args.mode:
-        return train(args, True, local_rank, data, Log_file, cfg, users_per_pass, model_dir, bert_state_dict=state)
+        return train(args, use_modal, local_rank, data, Log_file, cfg, users_per_pass, model_dir, bert_state_dict=state)
     if 'test' in args.mode:
-        return test(args, True, local_rank, data, Log_file, cfg, state, model_dir)
+        return test(args, use_modal, local_rank, data, Log_file, cfg, state, model_dir)
 
 
 if __name__ == "__main__":

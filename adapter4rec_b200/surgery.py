@@ -8,6 +8,10 @@ from .model.model import (BertAdaptedParallelSelfOutput, BertAdaptedSelfOutput, 
                           SASRecPfeifferVer2AdaptedSelfOutput, SoftEmbedding)
 
 
+ID_TOWER_ADAPTERS = ("item_tower 'id' has no item-encoder body to insert adapters into: use --adding_adapter_to None "
+                     "(an id run trains the embedding table and the user encoder, --fine_tune_to all)")
+
+
 def freeze_all(model):
     """fine_tune_to = 'None' (run.py:368-371)."""
     for _, param in model.named_parameters():
@@ -19,6 +23,8 @@ def insert_adapters(model, args, log=None):
     (run.py:389-452; SURVEY.md Appendix B-2).  New modules are trainable by default."""
     if 'None' in getattr(args, "adding_adapter_to", "bert"):
         return model
+    if not getattr(model, "use_modal", True):
+        raise ValueError(ID_TOWER_ADAPTERS)
     bert = model.bert_encoder.text_encoders.title.bert_model
     layers = bert.encoder.layer
     blocks = model.user_encoder.transformer_encoder.transformer_blocks
@@ -88,6 +94,8 @@ def insert_adapters_cv(model, args):
                            VITCompacterAdaptedOutput, VITCompacterAdaptedSelfOutput)
     if 'None' in getattr(args, "adding_adapter_to", "all"):
         return model
+    if not getattr(model, "use_modal", True):
+        raise ValueError(ID_TOWER_ADAPTERS)
     net = model.cv_encoder.image_net
     layers = net.vit.encoder.layer
     blocks = model.user_encoder.transformer_encoder.transformer_blocks

@@ -441,10 +441,35 @@ A4R_API int a4r_gather_rows(const void* table, const int64_t* ids, void* out, in
  *   [B, S1] int64 negatives to use instead (replay / parity against the reference's Python RNG).
  * Draw a of slot (b, j) is a pure function of (seed, offset + (b*S1 + j)*64 + a): a caller advances offset by
  * B*S1*64 per batch.  All pointers are device pointers; item_content and out 16-byte aligned, W even.
+ * Ids-only mode (item_content = NULL, W = 0, out may be NULL): the id item tower's sample (BuildTrainDataset with
+ * use_modal = False returns the ids [S1, 2] themselves) is [seqs | neg_out]; only log_mask and neg_out are written, and
+ * neg_out is exactly what the full call returns for the same (seed, offset).
  * ------------------------------------------------------------------------------------------------ */
 A4R_API int a4r_sample_train_batch(const int64_t* seqs, const int64_t* item_content, const int64_t* neg_in, int64_t* out,
                                    float* log_mask, int64_t* neg_out, int32_t* fail_flag, int64_t B, int64_t S1, int64_t W,
                                    int64_t item_num, uint64_t seed, uint64_t offset, a4r_stream_t stream);
+
+/* ------------------------------------------------------------------------------------------------
+ * ID item tower (--item_tower id): nn.Embedding(item_num + 1, D, padding_idx=0) reached from Model.forward
+ * (`input_embs_all = self.id_embedding(sample_items)`, the use_modal = False branch of Downstream/Text/model/model.py's
+ * Model / ModelCPC and of Downstream/CV/model/model.py's), forward and backward.
+ *
+ * a4r_id_embed_fwd: ids int64 [B, S1, 2] (S1 = max_seq_len + 1), table f32 [V, D] (the fp32 master, 16-byte aligned,
+ *   D %% 4 == 0) -> emb bf16 [B, S1, 2, D] = bf16_rne(table[ids]) and, if hist != NULL, hist bf16 [B, S1-1, D] =
+ *   emb[:, :S1-1, 0] (the user-encoder input).  An id outside [0, V) reads as a zero row.  No bf16 copy of the table is
+ *   made: the traffic is the gathered rows only.
+ * a4r_id_embed_bwd: the table gradient of both outputs.  sorted_ids [R] / order [R] (R = B*S1*2) are a STABLE ascending
+ *   sort of the flat ids (order = the flat occurrence index of each sorted entry).  For every id in [0, V) other than
+ *   padding_idx that occurs, row id of grad f32 [V, D] receives the fp32 sum of its occurrences r in ascending r, where
+ *   occurrence r = (b, j, t) contributes d_emb[r] and then, if t == 0 and j < S1-1 and d_hist != NULL, d_hist[b, j]
+ *   (d_emb bf16 [B, S1, 2, D], d_hist bf16 [B, S1-1, D]); grad[id] = sum (accumulate = 0) or grad[id] + sum
+ *   (accumulate = 1).  Rows of ids that do not occur are not touched.  No atomics: bit-identical run to run.
+ * ------------------------------------------------------------------------------------------------ */
+A4R_API int a4r_id_embed_fwd(const float* table, int64_t V, int64_t D, const int64_t* ids, int64_t B, int64_t S1,
+                             void* emb, void* hist, a4r_stream_t stream);
+A4R_API int a4r_id_embed_bwd(const int64_t* sorted_ids, const int64_t* order, const void* d_emb, const void* d_hist,
+                             float* grad, int64_t V, int64_t D, int64_t B, int64_t S1, int64_t padding_idx,
+                             int32_t accumulate, a4r_stream_t stream);
 
 /* ------------------------------------------------------------------------------------------------
  * K11 + K12: full-ranking scores fused with the history mask and per-user top-k.

@@ -1,11 +1,12 @@
 """-m gpu: counter-based dropout (train-mode semantics of nn.Dropout in the reference's BERT / SASRec blocks).
-The RNG is restated on the host (splitmix64) so the kernels can be checked against torch with the SAME mask."""
+The RNG is restated on the host (tests/dropout_rng.py) so the kernels can be checked against torch with the SAME mask."""
 import os
 import sys
 
-import numpy as np
 import pytest
 import torch
+
+import dropout_rng as R
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, os.path.join(HERE, "golden"))
@@ -13,24 +14,11 @@ sys.path.insert(0, os.path.join(os.path.dirname(HERE), "oracle"))
 
 pytestmark = pytest.mark.gpu
 BF16 = torch.bfloat16
-M64 = (1 << 64) - 1
-
-
-def rng64(seed, counter):
-    """host restatement of rng64() in csrc/a4r_common.cuh (splitmix64 finaliser)"""
-    z = (counter.astype(np.uint64) * np.uint64(0x9E3779B97F4A7C15) + np.uint64(seed))
-    z = (z ^ (z >> np.uint64(30))) * np.uint64(0xBF58476D1CE4E5B9)
-    z = (z ^ (z >> np.uint64(27))) * np.uint64(0x94D049BB133111EB)
-    return z ^ (z >> np.uint64(31))
 
 
 def keep_mask(seed, offset, n, p):
-    """mask of n consecutive elements starting at counter `offset` (4 elements per counter)"""
-    thr = int(p * 65536.0 + 0.5)
-    with np.errstate(over="ignore"):
-        bits = rng64(seed, np.arange((n + 3) // 4, dtype=np.uint64) + np.uint64(offset))
-    lanes = np.stack([(bits >> np.uint64(16 * k)) & np.uint64(0xFFFF) for k in range(4)], 1).reshape(-1)[:n]
-    return torch.from_numpy((lanes >= thr).astype(np.float32)), 65536.0 / (65536 - thr)
+    """f32 mask of n consecutive elements starting at counter `offset` (4 elements per counter), and the kept scale"""
+    return R.element_keep(seed, offset, p, torch.zeros(1, dtype=torch.int64), n)[0].float(), R.keep_scale(p)
 
 
 def test_dropout_kernel_matches_host_rng_and_is_unbiased():
@@ -66,38 +54,47 @@ def test_dropout_add_function_backward_reuses_the_mask():
 
 @pytest.mark.parametrize("N,L,heads,dh,causal", [(6, 30, 12, 64, False), (9, 20, 2, 32, True)])
 def test_attention_probability_dropout(N, L, heads, dh, causal):
+    """probability dropout of the short-sequence kernel, without and with a key mask (BERT: the int64 [ids | mask] right
+    half, right-padded; SASRec: f32, left-padded; both with a fully masked row)"""
     from adapter4rec_b200 import ops
     H = heads * dh
     g = torch.Generator(device="cuda").manual_seed(3)
     qkv = torch.randn((N * L, 3 * H), generator=g, device="cuda").to(BF16)
     dctx = torch.randn((N * L, H), generator=g, device="cuda").to(BF16)
     p, seed, off = 0.1, 4242, 1000
-    # mask[n, h, i, j] with nt = j/8, t = (j%8)/2, e = j%2:
-    #   lane ((nt&1)*2 + e) of rng64(seed, off + ((n*heads + h)*32 + i)*8 + (nt>>1)*4 + t)      (attention_small.cu)
-    n_i, h_i, i_i, j_i = np.meshgrid(np.arange(N), np.arange(heads), np.arange(L), np.arange(L), indexing="ij")
-    nt, tt, ee = j_i // 8, (j_i % 8) // 2, j_i % 2
-    ctr = (off + ((n_i * heads + h_i) * 32 + i_i) * 8 + (nt >> 1) * 4 + tt).astype(np.uint64)
-    with np.errstate(over="ignore"):
-        bits = rng64(seed, ctr)
-    lane = (bits >> (16 * ((nt & 1) * 2 + ee)).astype(np.uint64)) & np.uint64(0xFFFF)
-    thr = int(p * 65536.0 + 0.5)
-    mask = torch.from_numpy((lane >= thr).astype(np.float32)).cuda()
-    scale = 65536.0 / (65536 - thr)
-    qf = qkv.float().requires_grad_(True)
-    q, k, v = [t.view(N, L, heads, dh).transpose(1, 2) for t in qf.view(N * L, 3, H).unbind(1)]
-    s = (q @ k.transpose(-1, -2)) * dh ** -0.5
+    keep = R.prob_keep(seed, off, p, torch.arange(N, device="cuda"), heads, L).float()
+    lens = torch.randint(1, L + 1, (N,), generator=g, device="cuda")
+    lens[1] = 0
+    ok = torch.arange(L, device="cuda")[None, :] < lens[:, None]
     if causal:
-        s = s + torch.where(torch.tril(torch.ones(L, L, dtype=torch.bool, device="cuda")), 0.0, -1e9)
-    ref = ((torch.softmax(s, -1) * mask * scale) @ v).transpose(1, 2).reshape(N * L, H)
-    got = ops.attn_small_fwd(qkv, N, L, heads, dh, causal=causal, mask_neg=-1e9, dropout=(p, seed, off))
-    err = (got.float() - ref.detach()).abs()
-    assert bool((err <= 2e-2 + 2 ** -6 * ref.detach().abs()).all()), float(err.max())
-    ref.backward(dctx.float())
-    dqkv = ops.attn_small_bwd(qkv, dctx, N, L, heads, dh, causal=causal, mask_neg=-1e9, dropout=(p, seed, off))
-    for j, nm in enumerate(("dq", "dk", "dv")):
-        a, b = dqkv[:, j * H:(j + 1) * H].float(), qf.grad[:, j * H:(j + 1) * H]
-        rel = float((a - b).norm() / b.norm())
-        assert rel <= 2e-2, "%s relative L2 error %.4f" % (nm, rel)
+        ok = ok.flip(1)
+        masks = [(None, None), (ok, ok.float())]
+    else:
+        both = torch.zeros((N, 2 * L), dtype=torch.int64, device="cuda")
+        both[:, L:] = ok.long()
+        masks = [(None, None), (ok, both[:, L:])]
+    mask_neg = -1e9
+    for key_ok, mask in masks:
+        qf = qkv.float().requires_grad_(True)
+        q, k, v = [t.view(N, L, heads, dh).transpose(1, 2) for t in qf.view(N * L, 3, H).unbind(1)]
+        s = (q @ k.transpose(-1, -2)) * dh ** -0.5
+        allowed = torch.ones(N, 1, L, L, dtype=torch.bool, device="cuda")
+        if key_ok is not None:
+            allowed = allowed & key_ok.view(N, 1, 1, L)
+        if causal:
+            allowed = allowed & torch.tril(torch.ones(L, L, dtype=torch.bool, device="cuda"))
+        s = s + torch.where(allowed, 0.0, mask_neg)
+        ref = ((torch.softmax(s, -1) * keep * R.keep_scale(p)) @ v).transpose(1, 2).reshape(N * L, H)
+        got = ops.attn_small_fwd(qkv, N, L, heads, dh, mask=mask, causal=causal, mask_neg=mask_neg, dropout=(p, seed, off))
+        err = (got.float() - ref.detach()).abs()
+        assert bool((err <= 2e-2 + 2 ** -6 * ref.detach().abs()).all()), (mask is not None, float(err.max()))
+        ref.backward(dctx.float())
+        dqkv = ops.attn_small_bwd(qkv, dctx, N, L, heads, dh, mask=mask, causal=causal, mask_neg=mask_neg,
+                                  dropout=(p, seed, off))
+        for j, nm in enumerate(("dq", "dk", "dv")):
+            a, b = dqkv[:, j * H:(j + 1) * H].float(), qf.grad[:, j * H:(j + 1) * H]
+            rel = float((a - b).norm() / b.norm())
+            assert rel <= 2e-2, "%s relative L2 error %.4f (key mask: %s)" % (nm, rel, mask is not None)
 
 
 def test_train_mode_step_is_deterministic_given_the_seed_and_close_to_eval():
@@ -129,22 +126,30 @@ def test_train_mode_step_is_deterministic_given_the_seed_and_close_to_eval():
 
 
 @pytest.mark.parametrize("after", [False, True])
-def test_gemm_epilogue_dropout_before_and_after_the_residual(after):
-    """a4r_gemm_bf16_tn LINEAR epilogue: dropout(acc + bias) + residual (forward of dense -> dropout -> + input) and
-    dropout(acc + residual) (dropout_after_residual: the gradient through a dropout whose input gradient is a sum),
-    against torch with the host-restated mask."""
+@pytest.mark.parametrize("block_n", [0, 64, 128, 256, 512])
+@pytest.mark.parametrize("M,N,K", [(1000, 768, 64), (333, 72, 40)])
+@pytest.mark.parametrize("bias", [False, True])
+@pytest.mark.parametrize("res2", [False, True])
+def test_gemm_epilogue_dropout_before_and_after_the_residual(after, block_n, M, N, K, bias, res2):
+    """a4r_gemm_bf16_tn LINEAR epilogue: dropout(acc + bias) + residual(s) (forward of dense -> dropout -> + input) and
+    dropout(acc + bias + residual(s)) (dropout_after_residual: the gradient through a dropout whose input gradient is a
+    sum), against torch with the host-restated mask, on every tile width (0 = the automatic choice) and a ragged shape
+    (partial row and column tiles), counter offsets below and past 2^32."""
     from adapter4rec_b200 import ops
     g = torch.Generator(device="cuda").manual_seed(3)
-    M, N, K, p = 1000, 768, 64, 0.1
+    p = 0.1
     a = (torch.randn((M, K), generator=g, device="cuda") * 0.5).to(BF16)
     w = (torch.randn((N, K), generator=g, device="cuda") * 0.2).to(BF16)
     res = torch.randn((M, N), generator=g, device="cuda").to(BF16)
-    seed, off = 0x1234567, 4096
-    out = ops.gemm(a, w, residual=res, dropout=(p, seed, off), dropout_after=after)
-    mask, scale = keep_mask(seed, off, M * N, p)
-    mask = mask.view(M, N).cuda()
-    acc = a.float() @ w.float().t()
-    ref = (acc + res.float()) * mask * scale if after else acc * mask * scale + res.float()
+    r2 = torch.randn((M, N), generator=g, device="cuda").to(BF16) if res2 else None
+    b = torch.randn((N,), generator=g, device="cuda") if bias else None
+    seed, off = 0x1234567, 4096 if bias else (1 << 32) + 12345
+    out = ops.gemm(a, w, bias=b, residual=res, residual2=r2, block_n=block_n, dropout=(p, seed, off), dropout_after=after)
+    mask = R.element_keep(seed, off, p, torch.arange(M, device="cuda"), N).float()
+    scale = R.keep_scale(p)
+    acc = a.float() @ w.float().t() + (b if bias else 0.0)
+    rsum = res.float() + (r2.float() if res2 else 0.0)
+    ref = (acc + rsum) * mask * scale if after else acc * mask * scale + rsum
     err = (out.float() - ref).abs()
     assert bool((err <= 1e-2 + 8e-3 * ref.abs()).all()), float(err.max())
     if after:   # dropped elements of the SUM are exactly zero

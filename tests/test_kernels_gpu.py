@@ -270,19 +270,22 @@ def test_bce_loss(B, S, D, cpc):
 
 
 def test_adam_matches_torch():
+    """torch.optim.Adam fed g · grad_scale, without and with weight decay (the reference's --l2_weight): the decay term is
+    added to the SCALED gradient"""
     ops = _ops()
     n = 100003
     p0 = _rand((n,), 1, 1, torch.float32)
-    p = p0.clone()
-    m, v = torch.zeros_like(p), torch.zeros_like(p)
-    ref = torch.nn.Parameter(p0.clone())
-    opt = torch.optim.Adam([ref], lr=1e-3)
-    for step in range(1, 4):
-        g = _rand((n,), 1, 10 + step, torch.float32)
-        ref.grad = g.clone()
-        opt.step()
-        ops.adam_step(p, g * 4, m, v, 1e-3, 0.9, 0.999, 1e-8, 0.0, step, grad_scale=0.25)
-    _close(p, ref.detach(), 1e-6, 1e-6, "adam")
+    for wd in (0.0, 0.01):
+        p = p0.clone()
+        m, v = torch.zeros_like(p), torch.zeros_like(p)
+        ref = torch.nn.Parameter(p0.clone())
+        opt = torch.optim.Adam([ref], lr=1e-3, weight_decay=wd)
+        for step in range(1, 4):
+            g = _rand((n,), 1, 10 + step, torch.float32)
+            ref.grad = g.clone()
+            opt.step()
+            ops.adam_step(p, g * 4, m, v, 1e-3, 0.9, 0.999, 1e-8, wd, step, grad_scale=0.25)
+        _close(p, ref.detach(), 1e-6, 1e-6, "adam weight_decay=%g" % wd)
 
 
 def test_adam_dev_is_bit_identical_to_adam_step():

@@ -65,15 +65,16 @@ A4R_DEVICE void prob_dropout(float (&s)[2][4][4], const AttnParams& p, int n, in
     }
 }
 
-// A tile in shared memory: ROWS x COLS bf16, row-major, 16-byte chunks XOR-swizzled by (row & 7) so that
-// ldmatrix (8 rows x 16 B) is bank-conflict free.  COLS is 32 or 64 (4 or 8 chunks per row).
+// A tile in shared memory: ROWS x COLS bf16, row-major, 16-byte chunks XOR-swizzled by the row so that ldmatrix
+// (8 rows x 16 B) is bank-conflict free.  COLS is 32, 64 or 128 (4, 8 or 16 chunks per row).
 template <int COLS>
 struct Tile {
   static constexpr int kChunks = COLS / 8;
   static constexpr int kBytes = LP * COLS * 2;
   A4R_DEVICE static uint32_t off(int row, int chunk) {
-    // 128 B rows: xor with row; 64 B rows: two rows share a 128 B bank line, so xor with row/2
-    const int x = COLS == 64 ? row : (row >> 1);
+    // 128 B rows: xor with row; 64 B rows: two rows share a 128 B bank line, so xor with row/2.  256 B rows: xor with
+    // row & 15, so 8 consecutive rows at one logical chunk land on 8 different (physical chunk & 7), i.e. bank groups.
+    const int x = COLS >= 64 ? row : (row >> 1);
     return static_cast<uint32_t>(row * COLS * 2 + (((chunk ^ x) & (kChunks - 1)) << 4));
   }
 };
@@ -487,11 +488,223 @@ __global__ void __launch_bounds__(WARPS_PER_CTA * 32) attn_bwd_kernel(const Attn
   }
 }
 
+// ---- head_dim 128 ------------------------------------------------------------------------------------------------
+// Scores, P and dS reduce over the head dimension and are computed once over all 128 columns, as above.  The output
+// contractions (ctx = P·V; dQ = dS·K, dK = dSᵀ·Q, dV = Pᵀ·dO) run in 64-column halves, one product at a time, and
+// each half is written to shared memory before the next starts, so one 2 x 8 x 4 fp32 accumulator is live instead of
+// three 2 x 16 x 4 ones.  Each half overwrites the half of the input tile its product consumed, so no staging tile is
+// added.  A warp stages 24 KB (forward: Q, K, V) or 36 KB (backward: Q, K, V, dO, P, dS); 2-warp CTAs let 4 forward or
+// 3 backward CTAs share an SM.
+constexpr int WARPS_128 = 2;
+
+// A fragments [k-step][m-tile] of a 32 x 32 bf16 operand staged as a [32][32] tile: A = X (TRANS false) or Xᵀ (true)
+template <bool TRANS>
+A4R_DEVICE void load_a32(uint32_t (&a)[2][2][4], uint32_t sX, int lane) {
+#pragma unroll
+  for (int ks = 0; ks < 2; ++ks)
+#pragma unroll
+    for (int mt = 0; mt < 2; ++mt) {
+      if constexpr (TRANS)
+        load_a_t<32>(a[ks][mt], sX, mt * 16, ks * 16, lane);
+      else
+        load_a<32>(a[ks][mt], sX, mt * 16, ks * 16, lane);
+    }
+}
+
+// acc = A·B[:, c0 .. c0+64): A is 32 x 32 (fragments [k-step][m-tile]), B a [k][n] tile of 128 columns
+A4R_DEVICE void mma_half(float (&acc)[2][8][4], const uint32_t (&a)[2][2][4], uint32_t sB, int c0, int lane) {
+#pragma unroll
+  for (int mt = 0; mt < 2; ++mt)
+#pragma unroll
+    for (int nt = 0; nt < 8; ++nt)
+#pragma unroll
+      for (int e = 0; e < 4; ++e) acc[mt][nt][e] = 0.0f;
+#pragma unroll
+  for (int ks = 0; ks < 2; ++ks)
+#pragma unroll
+    for (int np = 0; np < 4; ++np) {
+      uint32_t b[4];
+      load_b_kn<128>(b, sB, c0 + np * 16, ks * 16, lane);
+      const uint32_t b0[2] = {b[0], b[1]}, b1[2] = {b[2], b[3]};
+      mma_bf16_16816(acc[0][np * 2], a[ks][0], b0);
+      mma_bf16_16816(acc[0][np * 2 + 1], a[ks][0], b1);
+      mma_bf16_16816(acc[1][np * 2], a[ks][1], b0);
+      mma_bf16_16816(acc[1][np * 2 + 1], a[ks][1], b1);
+    }
+}
+
+// bf16 of a 32 x 64 accumulator into columns c0 .. c0+64 of a swizzled [32][128] tile
+A4R_DEVICE void half_to_tile(uint8_t* tile, const float (&acc)[2][8][4], int c0, int lane) {
+  const int g = lane >> 2, t = lane & 3;
+#pragma unroll
+  for (int mt = 0; mt < 2; ++mt)
+#pragma unroll
+    for (int nt = 0; nt < 8; ++nt) {
+      const int r0 = mt * 16 + g, col = c0 + nt * 8 + 2 * t;
+      *reinterpret_cast<uint32_t*>(tile + Tile<128>::off(r0, col >> 3) + (col & 7) * 2) =
+          pack_bf16x2(acc[mt][nt][0], acc[mt][nt][1]);
+      *reinterpret_cast<uint32_t*>(tile + Tile<128>::off(r0 + 8, col >> 3) + (col & 7) * 2) =
+          pack_bf16x2(acc[mt][nt][2], acc[mt][nt][3]);
+    }
+}
+
+// tile[:, c0 .. c0+64) = A·tile[:, c0 .. c0+64): the product reads only that half of B, then overwrites it
+A4R_DEVICE void product_half_inplace(const uint32_t (&a)[2][2][4], uint8_t* tile, int c0, int lane) {
+  float acc[2][8][4];
+  mma_half(acc, a, smem_u32(tile), c0, lane);
+  __syncwarp();
+  half_to_tile(tile, acc, c0, lane);
+}
+
+template <>
+__global__ void __launch_bounds__(WARPS_128 * 32) attn_fwd_kernel<128>(const AttnParams p) {
+  extern __shared__ __align__(128) uint8_t smem_attn[];
+  constexpr int DH = 128, TB = Tile<DH>::kBytes;
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  uint8_t* my = smem_attn + warp * 3 * TB;
+  const int64_t total = static_cast<int64_t>(p.N) * p.heads;
+  for (int64_t w = static_cast<int64_t>(blockIdx.x) * WARPS_128 + warp; w < total;
+       w += static_cast<int64_t>(gridDim.x) * WARPS_128) {
+    const int n = static_cast<int>(w / p.heads), h = static_cast<int>(w % p.heads);
+    const int64_t Hd = static_cast<int64_t>(p.heads) * DH;
+    const SeqSpan sq = seq_span(p, n);
+    const __nv_bfloat16* q = p.qkv + sq.row0 * p.ld_qkv + h * DH;
+    uint8_t *tQ = my, *tV = my + 2 * TB;
+    load_tile<DH>(tQ, q, p.ld_qkv, sq.L, lane);
+    load_tile<DH>(my + TB, q + Hd, p.ld_qkv, sq.L, lane);
+    load_tile<DH>(tV, q + 2 * Hd, p.ld_qkv, sq.L, lane);
+    const uint32_t km = build_keymask(p, sq, lane);
+    cp_async_wait_all();
+    __syncwarp();
+    float s[2][4][4];
+    scores_softmax<DH>(s, smem_u32(tQ), smem_u32(my + TB), p, sq.L, lane, km);
+    if (p.drop_thr16 != 0) prob_dropout(s, p, n, h, lane);
+    uint32_t pa[2][2][4];
+#pragma unroll
+    for (int ks = 0; ks < 2; ++ks)
+#pragma unroll
+      for (int mt = 0; mt < 2; ++mt) acc_to_a(pa[ks][mt], s[mt][2 * ks], s[mt][2 * ks + 1]);
+    // O = P·V, one half at a time, staged in place of the V half it consumed
+#pragma unroll 1
+    for (int c0 = 0; c0 < DH; c0 += 64) product_half_inplace(pa, tV, c0, lane);
+    __syncwarp();
+    store_tile<DH>(tV, p.out + sq.row0 * p.ld_out + h * DH, p.ld_out, sq.L, lane);
+    __syncwarp();
+  }
+}
+
+template <>
+__global__ void __launch_bounds__(WARPS_128 * 32) attn_bwd_kernel<128>(const AttnParams p) {
+  extern __shared__ __align__(128) uint8_t smem_attn[];
+  constexpr int DH = 128, TB = Tile<DH>::kBytes, PB = Tile<32>::kBytes;
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  uint8_t* my = smem_attn + warp * (4 * TB + 2 * PB);
+  const int64_t total = static_cast<int64_t>(p.N) * p.heads;
+  for (int64_t w = static_cast<int64_t>(blockIdx.x) * WARPS_128 + warp; w < total;
+       w += static_cast<int64_t>(gridDim.x) * WARPS_128) {
+    const int n = static_cast<int>(w / p.heads), h = static_cast<int>(w % p.heads);
+    const int64_t Hd = static_cast<int64_t>(p.heads) * DH;
+    const SeqSpan sq = seq_span(p, n);
+    const __nv_bfloat16* q = p.qkv + sq.row0 * p.ld_qkv + h * DH;
+    uint8_t *tQ = my, *tK = my + TB, *tV = my + 2 * TB, *tdO = my + 3 * TB, *tP = my + 4 * TB, *tdS = tP + PB;
+    load_tile<DH>(tQ, q, p.ld_qkv, sq.L, lane);
+    load_tile<DH>(tK, q + Hd, p.ld_qkv, sq.L, lane);
+    load_tile<DH>(tV, q + 2 * Hd, p.ld_qkv, sq.L, lane);
+    load_tile<DH>(tdO, p.dout + sq.row0 * p.ld_out + h * DH, p.ld_out, sq.L, lane);
+    const uint32_t km = build_keymask(p, sq, lane);
+    cp_async_wait_all();
+    __syncwarp();
+    const uint32_t sdO = smem_u32(tdO), sP = smem_u32(tP), sdS = smem_u32(tdS);
+    float s[2][4][4];
+    scores_softmax<DH>(s, smem_u32(tQ), smem_u32(tK), p, sq.L, lane, km);
+    // dP = dO·Vᵀ over all 128 columns
+    float dp[2][4][4];
+#pragma unroll
+    for (int mt = 0; mt < 2; ++mt)
+#pragma unroll
+      for (int nt = 0; nt < 4; ++nt)
+#pragma unroll
+        for (int e = 0; e < 4; ++e) dp[mt][nt][e] = 0.0f;
+#pragma unroll
+    for (int k0 = 0; k0 < DH; k0 += 16) {
+      uint32_t a0[4], a1[4];
+      load_a<DH>(a0, sdO, 0, k0, lane);
+      load_a<DH>(a1, sdO, 16, k0, lane);
+#pragma unroll
+      for (int np = 0; np < 2; ++np) {
+        uint32_t b[4];
+        load_b_nk<DH>(b, smem_u32(tV), np * 16, k0, lane);
+        const uint32_t b0[2] = {b[0], b[1]}, b1[2] = {b[2], b[3]};
+        mma_bf16_16816(dp[0][np * 2], a0, b0);
+        mma_bf16_16816(dp[0][np * 2 + 1], a0, b1);
+        mma_bf16_16816(dp[1][np * 2], a1, b0);
+        mma_bf16_16816(dp[1][np * 2 + 1], a1, b1);
+      }
+    }
+    // dropout and dS exactly as in the 32 / 64 kernel
+    float sd[2][4][4];
+#pragma unroll
+    for (int mt = 0; mt < 2; ++mt)
+#pragma unroll
+      for (int nt = 0; nt < 4; ++nt)
+#pragma unroll
+        for (int e = 0; e < 4; ++e) sd[mt][nt][e] = s[mt][nt][e];
+    if (p.drop_thr16 != 0) {
+      prob_dropout(sd, p, n, h, lane);
+#pragma unroll
+      for (int mt = 0; mt < 2; ++mt)
+#pragma unroll
+        for (int nt = 0; nt < 4; ++nt)
+#pragma unroll
+          for (int e = 0; e < 4; ++e) dp[mt][nt][e] = (sd[mt][nt][e] != 0.0f) ? dp[mt][nt][e] * p.drop_scale : 0.0f;
+    }
+#pragma unroll
+    for (int mt = 0; mt < 2; ++mt)
+#pragma unroll
+      for (int hh = 0; hh < 2; ++hh) {
+        float d = 0.0f;
+#pragma unroll
+        for (int nt = 0; nt < 4; ++nt)
+#pragma unroll
+          for (int e = 0; e < 2; ++e) d += s[mt][nt][hh * 2 + e] * dp[mt][nt][hh * 2 + e];
+        d += __shfl_xor_sync(0xffffffffu, d, 1);
+        d += __shfl_xor_sync(0xffffffffu, d, 2);
+#pragma unroll
+        for (int nt = 0; nt < 4; ++nt)
+#pragma unroll
+          for (int e = 0; e < 2; ++e)
+            dp[mt][nt][hh * 2 + e] = s[mt][nt][hh * 2 + e] * (dp[mt][nt][hh * 2 + e] - d) * p.scale;
+      }
+    acc_to_tile<32, 4>(tP, sd, 1.f, 1.f, 1.f, 1.f, lane);
+    acc_to_tile<32, 4>(tdS, dp, 1.f, 1.f, 1.f, 1.f, lane);
+    __syncwarp();
+    // V is no longer needed.  Each half of dQ = dS·K, dK = dSᵀ·Q, dV = Pᵀ·dO replaces the half of K, Q, dO it read.
+    // The A operands come back from the staged bf16 tiles: the same values the 32 / 64 kernel packs from registers.
+#pragma unroll 1
+    for (int c0 = 0; c0 < DH; c0 += 64) {
+      uint32_t a[2][2][4];
+      load_a32<false>(a, sdS, lane);
+      product_half_inplace(a, tK, c0, lane);
+      load_a32<true>(a, sdS, lane);
+      product_half_inplace(a, tQ, c0, lane);
+      load_a32<true>(a, sP, lane);
+      product_half_inplace(a, tdO, c0, lane);
+    }
+    __syncwarp();
+    __nv_bfloat16* dq = p.out + sq.row0 * p.ld_qkv + h * DH;
+    store_tile<DH>(tK, dq, p.ld_qkv, sq.L, lane);
+    store_tile<DH>(tQ, dq + Hd, p.ld_qkv, sq.L, lane);
+    store_tile<DH>(tdO, dq + 2 * Hd, p.ld_qkv, sq.L, lane);
+    __syncwarp();
+  }
+}
+
 int check_common(const a4r_attn_args* a) {
   A4R_CHECK_ARG(a != nullptr, "attention: args is NULL");
   A4R_CHECK_ARG(a->qkv && a->out, "attention: qkv/out must be non-NULL");
   A4R_CHECK_ARG(a->L >= 1 && a->L <= LP, "attention_small: L must be in [1,32] (got %lld)", (long long)a->L);
-  A4R_CHECK_ARG(a->head_dim == 32 || a->head_dim == 64, "attention_small: head_dim must be 32 or 64");
+  A4R_CHECK_ARG(a->head_dim == 32 || a->head_dim == 64 || a->head_dim == 128,
+                "attention_small: head_dim must be 32, 64 or 128 (got %lld)", (long long)a->head_dim);
   A4R_CHECK_ARG(a->heads >= 1 && a->N >= 0, "attention: bad heads/N");
   A4R_CHECK_ARG(a->ld_qkv >= 3 * a->heads * a->head_dim && a->ld_qkv % 8 == 0, "attention: bad ld_qkv");
   A4R_CHECK_ARG(a->ld_out >= a->heads * a->head_dim && a->ld_out % 8 == 0, "attention: bad ld_out");
@@ -527,17 +740,24 @@ AttnParams to_params(const a4r_attn_args* a) {
   return p;
 }
 
+// warps: warps per CTA.  per_sm: NULL caps the grid at 8 CTAs per SM; otherwise the resident CTAs per SM, found with the
+// occupancy calculator when the attribute is set, so that every warp of the grid-stride loop runs the same share.
 template <typename K>
-int launch(K kernel, int smem, const AttnParams& p, cudaStream_t stream, bool* attr_done) {
+int launch(K kernel, int smem, const AttnParams& p, cudaStream_t stream, bool* attr_done, int warps = WARPS_PER_CTA,
+           int* per_sm = nullptr) {
   if (!*attr_done) {
     A4R_CUDA_OK(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
+    if (per_sm != nullptr) {
+      A4R_CUDA_OK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(per_sm, kernel, warps * 32, smem));
+      if (*per_sm < 1) *per_sm = 1;
+    }
     *attr_done = true;
   }
   const int64_t total = static_cast<int64_t>(p.N) * p.heads;
-  int64_t blocks = (total + WARPS_PER_CTA - 1) / WARPS_PER_CTA;
-  const int64_t cap = static_cast<int64_t>(a4r_num_sms()) * 8;
+  int64_t blocks = (total + warps - 1) / warps;
+  const int64_t cap = static_cast<int64_t>(a4r_num_sms()) * (per_sm != nullptr ? *per_sm : 8);
   if (blocks > cap) blocks = cap;
-  kernel<<<static_cast<int>(blocks), WARPS_PER_CTA * 32, smem, stream>>>(p);
+  kernel<<<static_cast<int>(blocks), warps * 32, smem, stream>>>(p);
   A4R_LAUNCH_OK();
   a4r_count_launch(1);
   return A4R_OK;
@@ -550,7 +770,11 @@ extern "C" int a4r_attn_small_fwd(const a4r_attn_args* a, a4r_stream_t stream) {
   if (rc != A4R_OK) return rc;
   if (a->N == 0) return A4R_OK;
   const AttnParams p = to_params(a);
-  static bool done64 = false, done32 = false;
+  static bool done64 = false, done32 = false, done128 = false;
+  static int per_sm128 = 0;
+  if (a->head_dim == 128)
+    return launch(attn_fwd_kernel<128>, WARPS_128 * 3 * Tile<128>::kBytes, p, static_cast<cudaStream_t>(stream), &done128,
+                  WARPS_128, &per_sm128);
   if (a->head_dim == 64)
     return launch(attn_fwd_kernel<64>, WARPS_PER_CTA * 3 * Tile<64>::kBytes, p, static_cast<cudaStream_t>(stream), &done64);
   return launch(attn_fwd_kernel<32>, WARPS_PER_CTA * 3 * Tile<32>::kBytes, p, static_cast<cudaStream_t>(stream), &done32);
@@ -562,7 +786,11 @@ extern "C" int a4r_attn_small_bwd(const a4r_attn_args* a, a4r_stream_t stream) {
   A4R_CHECK_ARG(a->dout != nullptr && a4r_aligned16(a->dout), "attention bwd: dout missing or unaligned");
   if (a->N == 0) return A4R_OK;
   const AttnParams p = to_params(a);
-  static bool done64 = false, done32 = false;
+  static bool done64 = false, done32 = false, done128 = false;
+  static int per_sm128 = 0;
+  if (a->head_dim == 128)
+    return launch(attn_bwd_kernel<128>, WARPS_128 * (4 * Tile<128>::kBytes + 2 * Tile<32>::kBytes), p,
+                  static_cast<cudaStream_t>(stream), &done128, WARPS_128, &per_sm128);
   if (a->head_dim == 64)
     return launch(attn_bwd_kernel<64>, WARPS_PER_CTA * (4 * Tile<64>::kBytes + 2 * Tile<32>::kBytes), p,
                   static_cast<cudaStream_t>(stream), &done64);

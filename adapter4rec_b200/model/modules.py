@@ -75,15 +75,15 @@ class MultiHeadedAttention(nn.Module):
             params += [m.weight, m.bias, getattr(m, "lora_A", None), getattr(m, "lora_B", None)]
         qkv = Fn.QKVFunction.apply(x2, self._qkv_cache, *params)
         pd = self.self_attention.dropout.p if self.training else 0.0
-        if self.d_k in (32, 64):
+        w = self.kernel_width(self.d_k)
+        if w == self.d_k:
             ctx = Fn.attention(qkv, mask, B, S, self.n_heads, self.d_k, causal=self.causal, mask_neg=SASREC_MASK_NEG,
                                dropout_p=pd)
         else:
-            # narrow heads (K-adapter inside SASRec: d = 16, 2 heads -> d_k = 8): every head is zero-padded to the
-            # 32-wide slot the attention kernel handles (q·k and p·v are unchanged by zero columns) with the softmax
-            # temperature of the TRUE head width; pad / slice are pure data movement
-            assert self.d_k < 32, "head width %d: supported are <= 32 and 64" % self.d_k
-            h3, w = 3 * self.n_heads, 32
+            # other widths (the K-adapter inside SASRec: d = 16, 2 heads -> d_k = 8; D = 192 with 4 heads -> 48): every
+            # head is zero-padded to the next width the attention kernel handles (q·k and p·v are unchanged by zero
+            # columns) with the softmax temperature of the TRUE head width; pad / slice are pure data movement
+            h3 = 3 * self.n_heads
             qp = torch.nn.functional.pad(qkv.view(-1, h3, self.d_k), (0, w - self.d_k)).reshape(-1, h3 * w)
             cp = Fn.attention(qp, mask, B, S, self.n_heads, w, causal=self.causal, mask_neg=SASREC_MASK_NEG,
                               dropout_p=pd, scale=self.d_k ** -0.5)
@@ -95,6 +95,17 @@ class MultiHeadedAttention(nn.Module):
         assert extra is None
         o = self.fc(ctx)
         return adapter(Fn.dropout_add(o, None, p) if p > 0 else o, extra_residual=x2)
+
+    KERNEL_WIDTHS = (32, 64, 128)   # head widths the short-sequence attention kernel runs natively
+
+    @classmethod
+    def kernel_width(cls, d_k):
+        """the kernel width a d_k-wide head runs at: d_k itself if native, else the next native width (zero-padded)"""
+        for w in cls.KERNEL_WIDTHS:
+            if d_k <= w:
+                return w
+        raise AssertionError("head width %d: the attention kernel supports head widths up to 128 (natively 32, 64 and "
+                             "128; narrower heads are zero-padded to the next of these)" % d_k)
 
     causal = True    # User_Encoder's mask (encoders.py:24-28); KAdapterBlock runs the same block with an all-ones mask
 

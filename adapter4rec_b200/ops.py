@@ -151,7 +151,8 @@ def _attn_args(qkv, N, L, heads, head_dim, mask, causal, mask_neg, dropout=None,
 
 
 def _attn_kernel(L, head_dim, causal, direction):
-    """short-sequence kernel for L <= 32, the CTA-per-(sequence, head) kernel for 32 < L <= 256 (ViT)"""
+    """short-sequence kernel for L <= 32 (head_dim 32, 64 or 128), the CTA-per-(sequence, head) kernel for
+    32 < L <= 256 (ViT, head_dim 64)"""
     lib = _l.get_lib()
     if L <= 32:
         return (lib.a4r_attn_small_fwd if direction == "fwd" else lib.a4r_attn_small_bwd), "a4r_attn_small_" + direction
@@ -163,7 +164,8 @@ def _attn_kernel(L, head_dim, causal, direction):
 def attn_small_fwd(qkv, N, L, heads, head_dim, mask=None, causal=False, mask_neg=F32_MIN, want_lse=False, dropout=None,
                    scale=None, cu_seqlens=None):
     """returns ctx, or (ctx, lse) with want_lse (lse is None for the short-sequence kernel, which recomputes it).
-    cu_seqlens (int32 [N+1]): packed variable-length layout, L = the longest sequence (<= 32)."""
+    head_dim: 32, 64 or 128 for L <= 32; 64 for 32 < L <= 256.  Other widths are zero-padded by the caller
+    (model/modules.py).  cu_seqlens (int32 [N+1]): packed variable-length layout, L = the longest sequence (<= 32)."""
     assert qkv.dtype == BF16 and (cu_seqlens is not None or qkv.shape[0] == N * L)
     out = torch.empty((qkv.shape[0], heads * head_dim), dtype=BF16, device=qkv.device)
     a = _attn_args(qkv, N, L, heads, head_dim, mask, causal, mask_neg, dropout, scale, cu_seqlens)

@@ -114,7 +114,7 @@ typedef struct a4r_gemm_args {
 A4R_API int a4r_gemm_bf16_tn(const a4r_gemm_args* args, a4r_stream_t stream);
 
 /* ------------------------------------------------------------------------------------------------
- * K3: whole-sequence attention for short sequences (L <= 32; head_dim 32 or 64), forward / backward.
+ * K3: whole-sequence attention for short sequences (L <= 32; head_dim 32, 64 or 128), forward / backward.
  *
  * Replaces BertSelfAttention's softmax(q·kᵀ/√d + mask)·v (transformers, reached from
  * Downstream/Text/model/encoders.py:53) and SASRec's SelfAttention.forward

@@ -1,22 +1,21 @@
-// adapter_rows_sm100.cu — K5, third formulation: the Houlsby adapter block with NO staging transpose.
+// adapter_rows_sm100.cu — K5: the Houlsby adapter block in ONE pass over the hidden states.
 //
 //   a   = h + W_u · act(W_d · h + b_d) + b_u            AdapterBlock.forward, Downstream/Text/model/modules.py:131-134
 //   out = LayerNorm(a + input) | a + input | a          BertAdaptedSelfOutput.forward (model.py:292-297) / VITAdaptedOutput /
 //                                                       VITAdaptedSelfOutput (Downstream/CV/model/model.py:182-212)
 //
-// adapter_ln_sm100.cu moves every up-projection chunk TMEM -> registers -> fp32 staging tile -> registers so that the
-// epilogue threads can touch global memory in a coalesced (row-distributed) layout; measured, that skeleton alone costs
-// 20.6 us per 128-token tile against 13.4 us of HBM time (DESIGN.md §4.5).  Here every epilogue thread keeps the TMEM-native
-// layout (one token row per thread) from the accumulator to the result and ALL global traffic is TMA:
+// TMEM hands an epilogue thread one token ROW.  Every epilogue thread keeps that layout from the accumulator to the result and
+// ALL global traffic is TMA, so no staging transpose into a coalesced (row-distributed) layout is needed: measured, the
+// skeleton of a staged formulation alone cost 20.6 us per 128-token tile against 13.4 us of HBM time (DESIGN.md §4.5).
 //   warp 0   TMA producer of the down-projection operands (h k-blocks + W_d k-blocks, NSTAGE-deep ring);
 //   warp 20  TMA producer of W_u: 4 KB chunks ([32 output columns x 64] bf16) re-streamed from L2 for every tile through a ring
-//            of NWU slots.  (W_u used to be resident: 96 KB of the 227 KB, which left a 2-stage operand ring — a third of the
-//            tile time was the epilogue waiting for the NEXT tile's down-projection, 12 k-blocks at two DRAM round trips in
-//            flight.  Re-reading 96 KB per tile from L2 costs 1/8 more L2->SM traffic and frees the room for a 4-stage ring,
-//            a fourth residual box per group and double result boxes.)
+//            of NWU slots.  (Resident in shared memory, W_u would take 96 KB of the 227 KB and leave room for a 2-stage operand
+//            ring only — a third of the tile time was then the epilogue waiting for the NEXT tile's down-projection, 12 k-blocks
+//            at two DRAM round trips in flight.  Re-reading 96 KB per tile from L2 costs 1/8 more L2->SM traffic and frees the
+//            room for a 4-stage ring, a fourth residual box per group and double result boxes.)
 //   warp 1   tcgen05 issuer: S1 = h · W_dᵀ, then U = s · W_uᵀ in 32-column chunks, chunk c into TMEM stage c & 1;
 //   warps 2, 3  TMA producers of the RESIDUALS, one per epilogue group: [128 x 32] boxes of h and input (SWIZZLE_64B) through a
-//            ring of three single boxes per group (each ring has ONE consumer group: no cross-group barrier phases);
+//            ring of IN_BOXES single boxes per group (each ring has ONE consumer group: no cross-group barrier phases);
 //   warps 4-19 epilogue in two groups of 8 warps (chunk parity): residual rows from shared memory (conflict-free 16-byte
 //            reads), z = U + b_u + h + input in registers, then
 //              tail 1 / 2: bf16 row segment -> the warp's private 1 KB box -> TMA store (no barrier wider than a warp);
@@ -566,13 +565,33 @@ int make_tmap_box32(CUtensorMap* m, const void* base, int64_t rows, int64_t cols
 
 }  // namespace
 
-// shapes: H % 64 == 0, H == 768 fits the shared-memory plan (W_u resident); smaller H always fits
-bool a4r_adapter_rows_supported(int64_t H, int64_t r) {
-  return H % 64 == 0 && H >= 64 && H <= 768 && r % 8 == 0 && r >= 8 && r <= 64;
+// H <= 768: z parked as packed bf16 takes H / 2 <= 384 TMEM columns; r <= 64: the rank fits one k-block (RP)
+extern "C" int a4r_adapter_ln_supported(int64_t H, int64_t r) {
+  return (H % 64 == 0 && H >= 64 && H <= 768 && r % 8 == 0 && r >= 8 && r <= 64) ? 1 : 0;
 }
 
-// arguments are validated by the caller (a4r_adapter_ln_fwd)
-int a4r_adapter_rows_launch(const a4r_adapter_args* a, cudaStream_t stream) {
+extern "C" int a4r_adapter_ln_fwd(const a4r_adapter_args* a, a4r_stream_t stream) {
+  A4R_CHECK_ARG(a != nullptr, "adapter_ln: args is NULL");
+  A4R_CHECK_ARG(a->h && a->w_down && a->w_up && a->b_down && a->b_up && a->out, "adapter_ln: NULL pointer");
+  A4R_CHECK_ARG(a->M >= 0 && a->M < (1ll << 31), "adapter_ln: bad M");
+  A4R_CHECK_ARG(a4r_adapter_ln_supported(a->H, a->r), "adapter_ln: needs H %% 64 == 0, H <= 768, r %% 8 == 0, r <= 64 (H=%lld r=%lld)",
+                (long long)a->H, (long long)a->r);
+  A4R_CHECK_ARG(a->tail >= 0 && a->tail <= 2 && (a->act == 0 || a->act == 1), "adapter_ln: bad tail/act");
+  A4R_CHECK_ARG(a->lds == 0 || (a->lds >= a->r && a->lds % 8 == 0 && a->lds < (1 << 20)), "adapter_ln: bad lds");
+  A4R_CHECK_ARG(a->tail != 0 || (a->gamma && a->beta), "adapter_ln: tail 0 (LayerNorm) needs gamma and beta");
+  A4R_CHECK_ARG(a->tail == 2 || a->input != nullptr, "adapter_ln: tails 0 and 1 add `input`");
+  A4R_CHECK_ARG(a->ldh >= a->H && a->ldh % 8 == 0 && a4r_aligned16(a->h), "adapter_ln: bad h/ldh");
+  A4R_CHECK_ARG(a->input == nullptr || (a->ldi >= a->H && a->ldi % 8 == 0 && a4r_aligned16(a->input)), "adapter_ln: bad input/ldi");
+  A4R_CHECK_ARG(a4r_aligned16(a->w_down) && a4r_aligned16(a->w_up) && a4r_aligned16(a->out) && a4r_aligned16(a->b_up) &&
+                    (a->gamma == nullptr || (a4r_aligned16(a->gamma) && a4r_aligned16(a->beta))),
+                "adapter_ln: pointers must be 16B aligned");
+  A4R_CHECK_ARG((a->z_out == nullptr || a4r_aligned16(a->z_out)) && (a->s_out == nullptr || a4r_aligned16(a->s_out)) &&
+                    (a->u_out == nullptr || a4r_aligned16(a->u_out)),
+                "adapter_ln: optional outputs must be 16B aligned");
+  int rc = a4r_device_check();
+  if (rc != A4R_OK) return rc;
+  if (a->M == 0) return A4R_OK;
+
   RowParams p;
   p.b_down = a->b_down;
   p.b_up = a->b_up;
@@ -593,7 +612,6 @@ int a4r_adapter_rows_launch(const a4r_adapter_args* a, cudaStream_t stream) {
   p.eps = a->eps;
 
   CUtensorMap tmH, tmWd, tmWu, tmHr, tmIr, tmOut, tmZ;
-  int rc;
   if ((rc = a4r_make_tmap_bf16(&tmH, a->h, a->M, a->H, a->ldh, BM)) != A4R_OK) return rc;
   if ((rc = a4r_make_tmap_bf16(&tmWd, a->w_down, a->r, a->H, a->H, RP)) != A4R_OK) return rc;
   if ((rc = a4r_make_tmap_bf16(&tmWu, a->w_up, a->H, a->r, a->r, CC)) != A4R_OK) return rc;
@@ -616,7 +634,7 @@ int a4r_adapter_rows_launch(const a4r_adapter_args* a, cudaStream_t stream) {
   A4R_CUDA_OK(cudaFuncSetAttribute(adapter_rows_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem)));
   const int tiles = (p.M + BM - 1) / BM;
   const int grid = tiles < a4r_num_sms() ? tiles : a4r_num_sms();
-  adapter_rows_kernel<<<grid, THREADS, smem, stream>>>(tmH, tmWd, tmWu, tmHr, tmIr, tmOut, tmZ, p);
+  adapter_rows_kernel<<<grid, THREADS, smem, static_cast<cudaStream_t>(stream)>>>(tmH, tmWd, tmWu, tmHr, tmIr, tmOut, tmZ, p);
   A4R_LAUNCH_OK();
   a4r_count_launch(1);
   return A4R_OK;

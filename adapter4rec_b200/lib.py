@@ -62,7 +62,7 @@ class AdapterArgs(Structure):
         ("gamma", c_void_p), ("beta", c_void_p), ("out", c_void_p), ("z_out", c_void_p),
         ("mean", c_void_p), ("rstd", c_void_p), ("s_out", c_void_p), ("u_out", c_void_p),
         ("M", c_int64), ("H", c_int64), ("r", c_int64), ("act", c_int32), ("tail", c_int32), ("eps", c_float),
-        ("lds", c_int64), ("impl", c_int32),
+        ("lds", c_int64),
     ]
 
 
@@ -104,9 +104,6 @@ PROTOTYPES = {
     "a4r_dropout": (c_int32, [c_void_p, c_void_p, c_void_p, c_int64, c_float, ctypes.c_uint64, ctypes.c_uint64, c_void_p]),
     "a4r_colsum_workspace_bytes": (c_size_t, [c_int64]),
     "a4r_colsum": (c_int32, [c_void_p, c_int64, c_int64, c_int64, c_void_p, c_int32, c_void_p, c_size_t, c_void_p]),
-    "a4r_wgrad_workspace_bytes": (c_size_t, [c_int64, c_int64, c_int64]),
-    "a4r_wgrad_bf16": (c_int32, [c_void_p, c_int64, c_void_p, c_int64, c_void_p, c_int64, c_int64, c_int64, c_int64,
-                                 c_float, c_int32, c_void_p, c_size_t, c_void_p]),
     "a4r_wgrad_tc_workspace_bytes": (c_size_t, [c_int64, c_int64, c_int64]),
     "a4r_wgrad_tc_bf16": (c_int32, [c_void_p, c_int64, c_void_p, c_int64, c_void_p, c_int64, c_int64, c_int64, c_int64,
                                     c_float, c_int32, c_void_p, c_size_t, c_void_p]),

@@ -323,27 +323,9 @@ def colsum(x, width=None, out=None, accumulate=False):
     return out
 
 
-def wgrad_mma_sync(a, b, alpha=1.0, out=None, accumulate=False, n=None, k=None):
-    """dW[N,K] (+)= alpha * a[:, :N].T @ b[:, :K]   (a = dY [M,>=N], b = X [M,>=K]; fp32 result) on the round-1
-    mma.sync split-M kernel (a4r_wgrad_bf16).  Kept as an ABI entry point and as the cross-check of the tcgen05 kernel
-    in the tests; the product path (`wgrad` below) is the tcgen05 kernel."""
-    assert a.dtype == BF16 and b.dtype == BF16 and a.shape[0] == b.shape[0]
-    M = a.shape[0]
-    N = a.shape[1] if n is None else n
-    K = b.shape[1] if k is None else k
-    if out is None:
-        out = torch.empty((N, K), dtype=torch.float32, device=a.device)
-        accumulate = False
-    assert out.dtype == torch.float32 and tuple(out.shape) == (N, K) and out.stride(1) == 1
-    wsb = _l.get_lib().a4r_wgrad_workspace_bytes(M, N, K)
-    ws = workspace(wsb, a.device)
-    _l.check(_l.get_lib().a4r_wgrad_bf16(_p(a), _rows2d(a, "a"), _p(b), _rows2d(b, "b"), _p(out), out.stride(0), M, N, K,
-                                         float(alpha), int(accumulate), _p(ws), wsb, _stream()), "a4r_wgrad_bf16")
-    return out
-
-
-def wgrad_tc(a, b, alpha=1.0, out=None, accumulate=False, n=None, k=None):
-    """dW[N,K] (+)= alpha * a[:, :N].T @ b[:, :K] on tcgen05 (MN-major operands, split over tokens, fp32 result)."""
+def wgrad(a, b, alpha=1.0, out=None, accumulate=False, n=None, k=None):
+    """dW[N,K] (+)= alpha * a[:, :N].T @ b[:, :K]   (a = dY [M,>=N], b = X [M,>=K]) on tcgen05 (MN-major operands, split
+    over tokens, fp32 result): every weight gradient of the path."""
     assert a.dtype == BF16 and b.dtype == BF16 and a.shape[0] == b.shape[0]
     M = a.shape[0]
     N = a.shape[1] if n is None else n
@@ -357,9 +339,6 @@ def wgrad_tc(a, b, alpha=1.0, out=None, accumulate=False, n=None, k=None):
     _l.check(_l.get_lib().a4r_wgrad_tc_bf16(_p(a), _rows2d(a, "a"), _p(b), _rows2d(b, "b"), _p(out), out.stride(0), M, N, K,
                                             float(alpha), int(accumulate), _p(ws), wsb, _stream()), "a4r_wgrad_tc_bf16")
     return out
-
-
-wgrad = wgrad_tc   # every weight gradient of the path: 2-5x faster than the mma.sync kernel at every shape measured
 
 
 def _bce_args(prec, emb, log_mask, pos, neg, loss, count, cpc):
@@ -406,8 +385,7 @@ def adapter_ln_supported(H, r):
     return bool(_l.get_lib().a4r_adapter_ln_supported(int(H), int(r)))
 
 
-def adapter_ln_fwd(h, inp, w_down, b_down, w_up, b_up, gamma=None, beta=None, eps=0.0, act="relu", tail=0, save=False,
-                   impl=0):
+def adapter_ln_fwd(h, inp, w_down, b_down, w_up, b_up, gamma=None, beta=None, eps=0.0, act="relu", tail=0, save=False):
     """K5 in one kernel: out = tail(h + W_u act(W_d h + b_d) + b_u [+ inp]); tail 0 = LayerNorm, 1 = +inp, 2 = nothing.
     returns (out, z, mean, rstd, s, u): with save=True the tensors the backward reads (z/mean/rstd for tail 0, s always,
     u = pre-activation for GELU), else None.  s is a [M, r] VIEW of a [M, r + 16] buffer (32-byte aligned rows) whose column r holds ones
@@ -440,7 +418,6 @@ def adapter_ln_fwd(h, inp, w_down, b_down, w_up, b_up, gamma=None, beta=None, ep
                                                                          _p(rstd), _p(s), _p(u))
     a.M, a.H, a.r, a.act, a.tail, a.eps = M, H, r, {"relu": 0, "gelu": 1}[act], int(tail), float(eps)
     a.lds = 0 if s is None else s.stride(0)
-    a.impl = int(impl)       # 0 = default, 2 = staged kernel, 3 = row-per-thread kernel (include/adapter4rec.h)
     _l.check(_l.get_lib().a4r_adapter_ln_fwd(ctypes.byref(a), _stream()), "a4r_adapter_ln_fwd")
     return out, z, mean, rstd, s, u
 

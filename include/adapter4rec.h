@@ -208,9 +208,6 @@ A4R_API int a4r_layernorm_bwd_add(const void* dy, const void* z, const float* me
  * [r, r + 8) of every row, so that ONE weight-gradient GEMM dzᵀ·[s | 1] yields d(fc_up.weight) and d(fc_up.bias) together.
  * Shapes: H %% 64 == 0, H <= 768, r %% 8 == 0, r <= 64 (a4r_adapter_ln_supported); other shapes compose
  * a4r_gemm_bf16_tn + a4r_layernorm_fwd.
- * impl selects the kernel formulation explicitly (no environment variables, no process state): 0 = default (the
- * row-per-thread TMA kernel where the shape allows it, else the staged kernel), 2 = staged kernel, 3 = row-per-thread kernel
- * (A4R_EINVAL if the shape is outside a4r_adapter_rows_supported).  Both formulations produce the same tensors.
  * ------------------------------------------------------------------------------------------------ */
 typedef struct a4r_adapter_args {
   const void* h;
@@ -234,7 +231,6 @@ typedef struct a4r_adapter_args {
   int32_t tail;
   float eps;
   int64_t lds;
-  int32_t impl;
 } a4r_adapter_args;
 A4R_API int a4r_adapter_ln_supported(int64_t H, int64_t r);
 A4R_API int a4r_adapter_ln_fwd(const a4r_adapter_args* args, a4r_stream_t stream);
@@ -327,22 +323,15 @@ A4R_API int a4r_colsum(const void* x, int64_t ld, int64_t M, int64_t width, floa
                void* workspace, size_t workspace_bytes, a4r_stream_t stream);
 
 /* ------------------------------------------------------------------------------------------------
- * Weight gradient of a TRAINABLE low-rank module:  dW[N,K] (+)= alpha * A[M,N]ᵀ · B[M,K]   (f32 out)
+ * Weight gradient:  dW[N,K] (+)= alpha * A[M,N]ᵀ · B[M,K]   (f32 out)
  *
  * A = dY (bf16 [M,lda]), B = X (bf16 [M,ldb]) gives nn.Linear's dW[out,in]: AdapterBlock.fc_down / fc_up
- * (Downstream/Text/model/modules.py:117-127) and loralib's lora_B = dYᵀ·(x·Aᵀ), lora_A = (dY·B)ᵀ·x
- * (Downstream/Text/run.py:414-428).  One of N, K is small (<= 64): HBM-bound, deterministic split-M.
+ * (Downstream/Text/model/modules.py:117-127), loralib's lora_B = dYᵀ·(x·Aᵀ), lora_A = (dY·B)ᵀ·x
+ * (Downstream/Text/run.py:414-428) and, under full fine-tuning, every nn.Linear weight of the encoder when
+ * fine_tune_to = all (Pretraining/Text/run.py:241-253, Downstream/Text/run.py:372-376).
+ * tcgen05 with MN-major operand descriptors (the activations are read in place, no transposes), split over the token axis
+ * with a fixed-order reduction (deterministic).  N, K multiples of 8, dW 16-byte aligned, ldw % 4 == 0.
  * ------------------------------------------------------------------------------------------------ */
-A4R_API size_t a4r_wgrad_workspace_bytes(int64_t M, int64_t N, int64_t K);
-A4R_API int a4r_wgrad_bf16(const void* A, int64_t lda, const void* B, int64_t ldb, float* dW, int64_t ldw, int64_t M,
-                   int64_t N, int64_t K, float alpha, int32_t accumulate, void* workspace, size_t workspace_bytes,
-                   a4r_stream_t stream);
-
-/* The same contraction on tcgen05 (MN-major operand descriptors: the activations are read in place, no transposes),
- * split over the token axis with a fixed-order reduction: dW[N,K] (+)= alpha * A[M,N]^T . B[M,K], any N, K multiple of 8.
- * Serves full fine-tuning — every nn.Linear weight of the encoder when fine_tune_to = all
- * (Pretraining/Text/run.py:241-253, Downstream/Text/run.py:372-376) — and the skinny LoRA / adapter gradients.
- * dW 16-byte aligned, ldw % 4 == 0. */
 A4R_API size_t a4r_wgrad_tc_workspace_bytes(int64_t M, int64_t N, int64_t K);
 A4R_API int a4r_wgrad_tc_bf16(const void* A, int64_t lda, const void* B, int64_t ldb, float* dW, int64_t ldw, int64_t M,
                               int64_t N, int64_t K, float alpha, int32_t accumulate, void* workspace,

@@ -216,7 +216,7 @@ def test_embed_ln(roberta, prompt):
     _close(out, ref, 2 ** -6, 3e-2, "embed+ln")
 
 
-def test_act_bwd_colsum_wgrad():
+def test_act_bwd_colsum():
     ops = _ops()
     dy, u = _rand((1000, 64), 1, 1), _rand((1000, 64), 1.5, 2)
     uf = u.float().requires_grad_(True)
@@ -229,17 +229,6 @@ def test_act_bwd_colsum_wgrad():
     for M, W in ((40960, 64), (4104, 16), (4097, 64)):      # narrow: rows folded 16 / 8 / 1 at a time
         xn = _rand((M, W), 1, 6)
         _close(ops.colsum(xn), xn.float().sum(0), 1e-4, 2e-2, "colsum narrow %dx%d" % (M, W))
-    for (M, N, K) in [(5000, 768, 8), (3001, 8, 768), (4096, 768, 64), (777, 64, 768), (10240, 64, 16), (100, 16, 64)]:
-        a, b = _rand((M, N), 1, 4), _rand((M, K), 1, 5)
-        ref = a.float().t() @ b.float()
-        got = ops.wgrad_mma_sync(a, b, alpha=0.5)
-        _close(got, 0.5 * ref, 1e-3, 2e-3 * math.sqrt(M), "wgrad %dx%dx%d" % (M, N, K))
-        got2 = ops.wgrad_mma_sync(a, b, alpha=0.5, out=got.clone(), accumulate=True)
-        _close(got2, ref, 1e-3, 4e-3 * math.sqrt(M), "wgrad accumulate")
-    # operands that are column slices of wider buffers (T = x·Aᵀ padded to 64 columns)
-    t = _rand((3000, 64), 1, 6)
-    dq = _rand((3000, 2304), 1, 7)
-    _close(ops.wgrad_mma_sync(dq[:, :768], t, k=8), dq[:, :768].float().t() @ t[:, :8].float(), 1e-3, 0.2, "wgrad sliced")
 
 
 @pytest.mark.parametrize("B,S,D,cpc", [(64, 20, 64, False), (7, 10, 256, False), (33, 20, 768, False), (16, 20, 64, True)])
@@ -396,26 +385,26 @@ def test_adapter_ln_fused(M, H, r, act, tail):
 @pytest.mark.parametrize("M,N,K", [(5000, 768, 8), (3001, 8, 768), (4096, 768, 64), (777, 64, 768), (10240, 64, 16),
                                    (100, 16, 64), (6400, 768, 768), (4100, 3072, 768), (2050, 768, 3072), (64, 128, 256),
                                    (63, 136, 264), (0, 64, 64), (20000, 2304, 64)])
-def test_wgrad_tc(M, N, K):
+def test_wgrad(M, N, K):
     """tcgen05 weight gradient (MN-major operands, split over tokens): dW = alpha * A^T B against fp32 torch on the same
-    bf16-rounded operands; tolerance = fp32 accumulation-order noise, sqrt(M)-scaled like the mma.sync kernel's test."""
+    bf16-rounded operands; tolerance = fp32 accumulation-order noise, sqrt(M)-scaled."""
     ops = _ops()
     a, b = _rand((M, N), 1, 4), _rand((M, K), 1, 5)
     ref = a.float().t() @ b.float()
-    got = ops.wgrad_tc(a, b, alpha=0.5)
-    _close(got, 0.5 * ref, 1e-3, 2e-3 * math.sqrt(max(M, 1)), "wgrad_tc %dx%dx%d" % (M, N, K))
-    got2 = ops.wgrad_tc(a, b, alpha=0.5, out=got.clone(), accumulate=True)
-    _close(got2, ref, 1e-3, 4e-3 * math.sqrt(max(M, 1)), "wgrad_tc accumulate")
-    assert torch.equal(ops.wgrad_tc(a, b, alpha=0.5), got), "fixed-order reduction must be deterministic"
+    got = ops.wgrad(a, b, alpha=0.5)
+    _close(got, 0.5 * ref, 1e-3, 2e-3 * math.sqrt(max(M, 1)), "wgrad %dx%dx%d" % (M, N, K))
+    got2 = ops.wgrad(a, b, alpha=0.5, out=got.clone(), accumulate=True)
+    _close(got2, ref, 1e-3, 4e-3 * math.sqrt(max(M, 1)), "wgrad accumulate")
+    assert torch.equal(ops.wgrad(a, b, alpha=0.5), got), "fixed-order reduction must be deterministic"
 
 
-def test_wgrad_tc_strided_operands():
+def test_wgrad_strided_operands():
     ops = _ops()
     t = _rand((3000, 64), 1, 6)
     dq = _rand((3000, 2304), 1, 7)
-    _close(ops.wgrad_tc(dq[:, :768], t, k=8), dq[:, :768].float().t() @ t[:, :8].float(), 1e-3, 0.2, "wgrad_tc sliced")
-    _close(ops.wgrad_tc(dq[:, 768:1536], dq[:, 1536:], n=768, k=768), dq[:, 768:1536].float().t() @ dq[:, 1536:].float(),
-           1e-3, 0.3, "wgrad_tc two column slices")
+    _close(ops.wgrad(dq[:, :768], t, k=8), dq[:, :768].float().t() @ t[:, :8].float(), 1e-3, 0.2, "wgrad sliced")
+    _close(ops.wgrad(dq[:, 768:1536], dq[:, 1536:], n=768, k=768), dq[:, 768:1536].float().t() @ dq[:, 1536:].float(),
+           1e-3, 0.3, "wgrad two column slices")
 
 
 def test_scatter_add_rows_matches_embedding_backward():
@@ -485,20 +474,17 @@ def _run_tool(*argv, timeout=600):
     assert r.returncode == 0 and r.stdout.strip().endswith("ALL OK"), (r.stdout[-1500:], r.stderr[-1500:])
 
 
-@pytest.mark.parametrize("impl", ["2", "3"])
-def test_adapter_block_both_formulations(impl):
-    """K5 has two kernels behind a4r_adapter_ln_fwd, selected by the explicit `impl` field of a4r_adapter_args: the
-    row-per-thread TMA kernel (3, the default; adapter_rows_sm100.cu) and the staged one (2; adapter_ln_sm100.cu).
-    tools/k5_check.py runs every tail x activation x save combination at M = 128 / 1,000 / 20,000 (ragged last tile, several
-    tiles per CTA) against torch."""
-    _run_tool("k5_check.py", impl)
+def test_adapter_block_matches_torch():
+    """K5 (a4r_adapter_ln_fwd, adapter_rows_sm100.cu): tools/k5_check.py runs every tail x activation x save combination at
+    M = 128 / 1,000 / 20,000 (ragged last tile, several tiles per CTA) against torch."""
+    _run_tool("k5_check.py")
 
 
 def test_adapter_block_at_the_benchmarked_row_counts():
-    """K5 (default formulation) at M = 161,280 (8.5 tiles per persistent CTA: C1 at 128 users per pass) and M = 645,120 (+ a
-    ragged 645,197): the multi-tile ring / phase path the benchmark runs, every row against torch fp32, both ViT tails, both
-    activations, save on and off."""
-    _run_tool("k5_check.py", "3", "--big", timeout=900)
+    """K5 at M = 161,280 (8.5 tiles per persistent CTA: C1 at 128 users per pass) and M = 645,120 (+ a ragged 645,197): the
+    multi-tile ring / phase path the benchmark runs, every row against torch fp32, both ViT tails, both activations, save on
+    and off."""
+    _run_tool("k5_check.py", "--big", timeout=900)
 
 
 def test_vit_attention_tcgen05_forward_and_backward():

@@ -1,6 +1,6 @@
-"""Correctness of one K5 formulation (argv[1] = 2 staged | 3 row-per-thread, passed to a4r_adapter_ln_fwd as `impl`) against
-torch: all tails, relu / gelu, save on / off, ragged M; `--big` adds the benchmarked row counts (M = 161,280 = 8.5 tiles per
-persistent CTA and M = 645,120 = 34 tiles per CTA: the multi-tile ring / phase path), checked on EVERY row in row blocks."""
+"""Correctness of K5 (a4r_adapter_ln_fwd) against torch: all tails, relu / gelu, save on / off, ragged M; `--big` adds the
+benchmarked row counts (M = 161,280 = 8.5 tiles per persistent CTA and M = 645,120 = 34 tiles per CTA: the multi-tile ring /
+phase path), checked on EVERY row in row blocks."""
 import os, sys
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import torch
@@ -19,7 +19,7 @@ def rnd(*s, sc=1.0, seed=0):
     return (torch.randn(*s, device="cuda", generator=g) * sc).to(torch.bfloat16)
 
 
-def check(M, impl, wd, wu, bd, bu, g, b, tails=(0, 1, 2), acts=("relu", "gelu"), saves=(False, True), blk=32768):
+def check(M, wd, wu, bd, bu, g, b, tails=(0, 1, 2), acts=("relu", "gelu"), saves=(False, True), blk=32768):
     ok = True
     h, inp = rnd(M, H, seed=M + 1), rnd(M, H, seed=M + 2)
     for tail in tails:
@@ -27,7 +27,7 @@ def check(M, impl, wd, wu, bd, bu, g, b, tails=(0, 1, 2), acts=("relu", "gelu"),
             for save in saves:
                 gg, bb = (g, b) if tail == 0 else (None, None)
                 out, z, mean, rstd, s, u = ops.adapter_ln_fwd(h, inp if tail != 2 else None, wd, bd, wu, bu, gg, bb, 1e-12, act=act,
-                                                              tail=tail, save=save, impl=impl)
+                                                              tail=tail, save=save)
                 torch.cuda.synchronize()
                 e = es = ez = em = 0.0
                 ones_ok = True
@@ -59,7 +59,6 @@ def check(M, impl, wd, wu, bd, bu, g, b, tails=(0, 1, 2), acts=("relu", "gelu"),
 
 
 def main():
-    impl = int(sys.argv[1]) if len(sys.argv) > 1 and sys.argv[1].isdigit() else 0
     big = "--big" in sys.argv
     wd, wu = rnd(r, H, sc=0.05, seed=3), rnd(H, r, sc=0.05, seed=4)
     gen = torch.Generator(device="cuda").manual_seed(9)
@@ -67,12 +66,12 @@ def main():
     g, b = torch.rand(H, device="cuda", generator=gen) + 0.5, torch.randn(H, device="cuda", generator=gen) * 0.1
     ok = True
     if big:
-        ok &= check(161280, impl, wd, wu, bd, bu, g, b)
-        ok &= check(645120, impl, wd, wu, bd, bu, g, b, acts=("relu",))
-        ok &= check(645120 + 77, impl, wd, wu, bd, bu, g, b, tails=(0,), acts=("gelu",), saves=(True,))
+        ok &= check(161280, wd, wu, bd, bu, g, b)
+        ok &= check(645120, wd, wu, bd, bu, g, b, acts=("relu",))
+        ok &= check(645120 + 77, wd, wu, bd, bu, g, b, tails=(0,), acts=("gelu",), saves=(True,))
     else:
         for M in (128, 1000, 20000):
-            ok &= check(M, impl, wd, wu, bd, bu, g, b)
+            ok &= check(M, wd, wu, bd, bu, g, b)
     print("ALL OK" if ok else "FAILED")
 
 

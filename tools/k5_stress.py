@@ -1,4 +1,4 @@
-"""Race stress of the default K5 formulation: the same launch repeated `trials` times at a benchmarked row count, every result
+"""Race stress of the K5 kernel: the same launch repeated `trials` times at a benchmarked row count, every result
 compared with ONE torch fp32 reference.  A data race between the epilogue's shared-memory reads and the TMA refill of the residual
 ring (fixed in round 2: adapter_rows_sm100.cu `loads_returned`) showed up in 1-3 % of such launches as a few rows of one warp
 carrying the NEXT ring box's bytes; tools/k5_debug.py explains such mismatches by brute-force search over the operands."""

@@ -3,7 +3,12 @@
 set -e
 cd "$(dirname "$0")/.."
 mkdir -p tools/variants
-objs=$(ls adapter4rec_b200/build/*.o | grep -v adapter_rows_sm100)
+# one object per source present: a stale object of a deleted source would define its symbols a second time
+objs=""
+for src in adapter4rec_b200/csrc/*.cu; do
+  name=$(basename "$src" .cu)
+  [ "$name" = adapter_rows_sm100 ] || objs="$objs adapter4rec_b200/build/$name.o"
+done
 for v in "$@"; do
   IFS=_ read ns nwu inb <<< "$v"
   nvcc -gencode arch=compute_100a,code=sm_100a -lineinfo -O3 -std=c++17 --extended-lambda -Xcompiler -fPIC -Xcompiler -fvisibility=hidden \

@@ -17,8 +17,8 @@ du = torch.randn(M, 4 * H, device="cuda").to(torch.bfloat16)
 for it in range(2):
     ctx = ops.attn_small_fwd(qkv, N, L, heads, dh, mask=mask, dropout=(0.1, 1234, 0))
     dq = ops.attn_small_bwd(qkv, dctx, N, L, heads, dh, mask=mask, dropout=(0.1, 1234, 0))
-    g1 = ops.wgrad_tc(qkv, t1)          # d(B_ext) = dqkv^T [T | 1]   (2304 x 64)
-    g2 = ops.wgrad_tc(t1, x)            # d(A_cat) = dT^T x           (64 x 768)
-    g3 = ops.wgrad_tc(du, x)            # full fine-tuning: d(W_1)    (3072 x 768)
+    g1 = ops.wgrad(qkv, t1)             # d(B_ext) = dqkv^T [T | 1]   (2304 x 64)
+    g2 = ops.wgrad(t1, x)               # d(A_cat) = dT^T x           (64 x 768)
+    g3 = ops.wgrad(du, x)               # full fine-tuning: d(W_1)    (3072 x 768)
 torch.cuda.synchronize()
 print("done")

@@ -8,7 +8,7 @@ import torch.nn as nn
 
 from .. import functional as Fn
 from .. import ops
-from ..model.layers import BF16, LayerNorm, Linear, to_2d_bf16
+from ..model.layers import BF16, LayerNorm, Linear, frozen_ffn_dense, to_2d_bf16
 
 
 class ViTConfigLite:
@@ -208,14 +208,11 @@ class ViTLayer(nn.Module):
         y, x1 = self.layernorm_after.forward_skip(x1)
         out = self.output
         wi = self.intermediate.dense
-        inner = out.self_output if hasattr(out, "self_output") else out
-        wf = getattr(inner, "dense", None)
-        frozen = wf is not None and not (wi.weight.requires_grad or wi.bias.requires_grad or
-                                         wf.weight.requires_grad or wf.bias.requires_grad)
-        if frozen and type(out) is ViTOutput:
-            return Fn.FFNFunction.apply(y, wi.weight, wi.bias, wf.weight, wf.bias, x1, wi._cache, wf._cache)
-        if frozen and hasattr(out, "forward_from_dense"):
-            h = Fn.FFNFunction.apply(y, wi.weight, wi.bias, wf.weight, wf.bias, None, wi._cache, wf._cache)
+        wf = frozen_ffn_dense(wi, out)
+        if wf is not None and type(out) is ViTOutput:
+            return Fn.frozen_block(y, x1, wf, intermediate=wi)
+        if wf is not None and hasattr(out, "forward_from_dense"):
+            h = Fn.frozen_block(y, None, wf, intermediate=wi)
             return to_2d_bf16(out.forward_from_dense(h, x1))
         return to_2d_bf16(out(self.intermediate(y), x1))
 

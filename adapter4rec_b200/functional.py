@@ -104,94 +104,96 @@ def linear(x, weight, bias, cache, act=None, residual=None, residual2=None):
     return LinearFunction.apply(x, weight, bias, residual, residual2, cache, act)
 
 
-class FFNFunction(torch.autograd.Function):
-    """Frozen BERT feed-forward: h = GELU(y Wiᵀ + bi) Wfᵀ + bf (+ residual).  The backward fuses GELU' into the epilogue
-    of the first data-gradient GEMM and the residual gradient into the second, and keeps only the pre-activation."""
-
-    @staticmethod
-    def forward(ctx, y, wi, bi, wf, bf, residual, cache_i, cache_f):
-        w1, _ = cache_i.get(wi)
-        w2, _ = cache_f.get(wf)
-        need = ctx.needs_input_grad[0] or ctx.needs_input_grad[5]
-        u = torch.empty((y.shape[0], w1.shape[0]), dtype=BF16, device=y.device) if need else None
-        f = ops.gemm(y, w1, bias=bi.detach(), epilogue=ops.EPI_GELU, aux=u)
-        h = ops.gemm(f, w2, bias=bf.detach(), residual=residual)
-        ctx.caches = (cache_i, cache_f)
-        ctx.has_res = residual is not None
-        ctx.res_is_input = residual is y
-        ctx.save_for_backward(u, wi, wf)
-        return h
-
-    @staticmethod
-    def backward(ctx, dh):
-        u, wi, wf = ctx.saved_tensors
-        dh = dh.contiguous()
-        _, w2t = ctx.caches[1].get(wf, need_t=True)
-        _, w1t = ctx.caches[0].get(wi, need_t=True)
-        du = ops.gemm(dh, w2t, epilogue=ops.EPI_DGELU, aux=u)
-        # when the residual IS the input (post-LN BERT: h = FFN(y) + y) its gradient is folded into the epilogue of the
-        # last data-gradient GEMM and nothing is returned for the residual slot (autograd would add them otherwise).
-        fold = ctx.has_res and ctx.res_is_input
-        dy = ops.gemm(du, w1t, residual=dh if fold else None) if ctx.needs_input_grad[0] else None
-        dres = dh if (ctx.has_res and not fold and ctx.needs_input_grad[5]) else None
-        return dy, None, None, None, None, dres, None, None
+def _frozen(dense, intermediate=None):
+    """F of a frozen block: ((W, b, cache),) of the dense Linear, or ((Wi, bi, ci), (Wf, bf, cf)) of the GELU FFN pair
+    intermediate -> dense.  Frozen weights need no gradient, so they travel in this tuple rather than as node inputs."""
+    return tuple((m.weight, m.bias, m._cache) for m in ((dense,) if intermediate is None else (intermediate, dense)))
 
 
-class PostLNBlockFunction(torch.autograd.Function):
-    """One frozen post-LN residual block of BERT in a single autograd node:
+def _ln_args(ln):
+    return (None, None, 0.0) if ln is None else (ln.weight, ln.bias, ln.eps)
 
-        out = LayerNorm(dropout(F(x)) + res)       F(x) = x Woᵀ + bo                      (attention.output: BertSelfOutput)
-                                                  F(x) = GELU(x Wiᵀ + bi) Wfᵀ + bf       (intermediate + output: BertOutput)
 
+def _needs(ctx, names):
+    """{argument name: needs a gradient} of a node whose forward takes the arguments `names` in this order"""
+    return dict(zip(names, ctx.needs_input_grad))
+
+
+def _frozen_fwd(x, F, res, rng, need_u):
+    """(dropout(F(x)) (+ res), u): dropout (rng = (p, seed, offset) or None) and the residual live in the epilogue of F's
+    last GEMM; u is the FFN pair's pre-activation (the GELU′ operand of the backward), kept when need_u, else None."""
+    ws = [cache.get(w)[0] for w, _, cache in F]
+    u = None
+    if len(F) == 2:
+        u = torch.empty((x.shape[0], ws[0].shape[0]), dtype=BF16, device=x.device) if need_u else None
+        x = ops.gemm(x, ws[0], bias=F[0][1].detach(), epilogue=ops.EPI_GELU, aux=u)
+    return ops.gemm(x, ws[-1], bias=F[-1][1].detach(), residual=res, dropout=rng), u
+
+
+def _frozen_bwd(dh, u, F, fold):
+    """dx of _frozen_fwd from dh, the gradient at F's output (already through the dropout).  GELU′ rides in the epilogue
+    of the first data-gradient GEMM; fold (the skip gradient when res is x, or None) in that of the last."""
+    wts = [cache.get(w, need_t=True)[1] for w, _, cache in F]
+    if len(F) == 2:
+        dh = ops.gemm(dh, wts[1], epilogue=ops.EPI_DGELU, aux=u)
+    return ops.gemm(dh, wts[0], residual=fold)
+
+
+def _dropout_rng(p, x, F):
+    """(p, seed, offset) of the dropout on F's output, or None when p == 0"""
+    return (float(p),) + DropoutState.draw((x.shape[0] * F[-1][0].shape[0] + 3) // 4) if p > 0 else None
+
+
+class FrozenBlockFunction(torch.autograd.Function):
+    """A frozen dense layer or FFN pair with its dropout, residual and post-LN LayerNorm in a single autograd node:
+
+        out = tail(dropout(F(x)) + res)       F(x) = x Woᵀ + bo                  (attention.output: BertSelfOutput)
+                                             F(x) = GELU(x Wiᵀ + bi) Wfᵀ + bf   (intermediate + output: BertOutput, ViTOutput)
+
+    tail = LayerNorm (gamma given; gamma / beta may be trainable: finetune_layernorm) or nothing (then p must be 0).
+    res = None, x itself (its gradient rides in the epilogue of the last data-gradient GEMM) or another tensor.
     Forward: dropout and the residual add live in the epilogue of the last GEMM (counter RNG).  Backward: LayerNorm's
-    backward kernel emits dz AND dz ⊙ mask/(1-p) (the gradient through the dropout) in one pass; GELU′ and the residual
-    gradient live in the epilogues of the data-gradient GEMMs.  Only LayerNorm may be trainable (finetune_layernorm)."""
+    backward kernel emits dz AND dz ⊙ mask/(1-p) (the gradient through the dropout) in one pass; GELU′ and the skip
+    gradient live in the epilogues of the data-gradient GEMMs."""
+
+    ARGS = ("x", "res", "gamma", "beta", "eps", "p", "F")
 
     @staticmethod
-    def forward(ctx, x, res, gamma, beta, eps, p, w1, b1, cache1, w2, b2, cache2):
-        ffn = w2 is not None
-        need = any(ctx.needs_input_grad[:4])
-        rng = (float(p),) + DropoutState.draw((x.shape[0] * (w2 if ffn else w1).shape[0] + 3) // 4) if p > 0 else None
-        wa, _ = cache1.get(w1)
-        u = None
-        if ffn:
-            wb, _ = cache2.get(w2)
-            u = torch.empty((x.shape[0], wa.shape[0]), dtype=BF16, device=x.device) if need else None
-            f = ops.gemm(x, wa, bias=b1.detach(), epilogue=ops.EPI_GELU, aux=u)
-            z = ops.gemm(f, wb, bias=b2.detach(), residual=res, dropout=rng)
-        else:
-            z = ops.gemm(x, wa, bias=b1.detach(), residual=res, dropout=rng)
-        g, b = gamma.detach().float().contiguous(), beta.detach().float().contiguous()
-        out, _, mean, rstd = ops.layernorm_fwd(z, g, b, eps, want_stats=need)
-        ctx.rng, ctx.ffn, ctx.caches = rng, ffn, (cache1, cache2)
-        ctx.res_is_input = res is x
-        if need:
-            ctx.save_for_backward(z, mean, rstd, g, u, w1, w2)
+    def forward(ctx, x, res, gamma, beta, eps, p, F):
+        assert gamma is not None or p == 0, "dropout without the LayerNorm tail is not fused"
+        need = any(_needs(ctx, FrozenBlockFunction.ARGS).values())
+        rng = _dropout_rng(p, x, F)
+        out, u = _frozen_fwd(x, F, res, rng, need)
+        ctx.rng, ctx.F, ctx.fold, ctx.ln = rng, F, res is x, gamma is not None
+        z = mean = rstd = g = None
+        if ctx.ln:
+            z, g, b = out, gamma.detach().float().contiguous(), beta.detach().float().contiguous()
+            out, _, mean, rstd = ops.layernorm_fwd(z, g, b, eps, want_stats=need)
+        ctx.save_for_backward(z, mean, rstd, g, u)
         return out
 
     @staticmethod
     def backward(ctx, dout):
-        z, mean, rstd, g, u, w1, w2 = ctx.saved_tensors
-        dout = dout.contiguous()
-        want_ln = ctx.needs_input_grad[2] or ctx.needs_input_grad[3]
-        dg = db = None
-        if want_ln:
-            dg, db = torch.empty_like(g), torch.empty_like(g)
-        r = ops.layernorm_bwd(dout, z, mean, rstd, g, dgamma=dg, dbeta=db, masked=ctx.rng)
-        dz, dzm = r if ctx.rng is not None else (r, r)
-        dx = None
-        if ctx.needs_input_grad[0]:
-            fold = dz if ctx.res_is_input else None      # res is x: the skip gradient rides in the last epilogue
-            if ctx.ffn:
-                _, w2t = ctx.caches[1].get(w2, need_t=True)
-                _, w1t = ctx.caches[0].get(w1, need_t=True)
-                du = ops.gemm(dzm, w2t, epilogue=ops.EPI_DGELU, aux=u)
-                dx = ops.gemm(du, w1t, residual=fold)
-            else:
-                _, w1t = ctx.caches[0].get(w1, need_t=True)
-                dx = ops.gemm(dzm, w1t, residual=fold)
-        dres = dz if (ctx.needs_input_grad[1] and not ctx.res_is_input) else None
-        return dx, dres, dg, db, None, None, None, None, None, None, None, None
+        z, mean, rstd, g, u = ctx.saved_tensors
+        need = _needs(ctx, FrozenBlockFunction.ARGS)
+        grads = {}
+        dout = dz = dzm = dout.contiguous()
+        if ctx.ln:
+            if need["gamma"] or need["beta"]:
+                grads["gamma"], grads["beta"] = torch.empty_like(g), torch.empty_like(g)
+            r = ops.layernorm_bwd(dout, z, mean, rstd, g, dgamma=grads.get("gamma"), dbeta=grads.get("beta"), masked=ctx.rng)
+            dz, dzm = r if ctx.rng is not None else (r, r)
+        if need["x"]:
+            grads["x"] = _frozen_bwd(dzm, u, ctx.F, dz if ctx.fold else None)
+        if need["res"] and not ctx.fold:
+            grads["res"] = dz
+        return tuple(grads.get(n) for n in FrozenBlockFunction.ARGS)
+
+
+def frozen_block(x, res, dense, intermediate=None, ln=None, p=0.0):
+    """tail(dropout(F(x)) + res) as one node (FrozenBlockFunction).  dense / intermediate: the block's frozen Linear
+    modules (intermediate None: F is dense alone); ln: its LayerNorm module, or None for no tail (p must then be 0)."""
+    return FrozenBlockFunction.apply(x, res, *_ln_args(ln), p, _frozen(dense, intermediate))
 
 
 class LayerNormFunction(torch.autograd.Function):
@@ -733,153 +735,83 @@ def inbatch_softmax_loss(prec, emb, item_ids, log_mask, cand_bias=None):
     return InbatchCeFunction.apply(prec, emb, item_ids, log_mask, cand_bias)
 
 
-class HoulsbyBlockFunction(torch.autograd.Function):
-    """K5 as one autograd node: out = tail(h + W_u act(W_d h + b_d) + b_u [+ inp]) with tail = LayerNorm (gamma given),
-    or nothing.  Forward = the fused a4r_adapter_ln_fwd kernel; backward = LayerNorm backward, two skinny data-gradient
-    GEMMs (act' and the skip gradient in their epilogues) and the rank-r weight / bias gradients — no torch arithmetic."""
+class AdapterBlockFunction(torch.autograd.Function):
+    """K5 as one autograd node, optionally behind a frozen dense layer or FFN pair F (the serial Houlsby wrapper of a
+    frozen post-LN block, BertAdaptedSelfOutput.forward, Downstream/Text/model/model.py:292-297):
+
+        h   = dropout(F(x)) when F is given, else x
+        out = tail(h + W_u act(W_d h + b_d) + b_u [+ inp])       tail = LayerNorm (gamma given), + inp, or nothing
+
+    Forward: F's GEMMs (dropout in the epilogue of the last one, counter RNG), then the fused a4r_adapter_ln_fwd kernel.
+    Backward: LayerNorm backward, two skinny data-gradient GEMMs and the rank-r weight / bias gradients.  The second GEMM
+    forms (ds W_d + dz) and, behind F, masks the SUM with the regenerated dropout mask in its epilogue
+    (`dropout_after_residual`), so no stand-alone dropout pass exists in either direction; GELU′ and — when `inp` is x
+    itself (the feed-forward block) — the skip gradient ride in the epilogues of F's data-gradient GEMMs.  Trainable: the
+    adapter and the LayerNorm; F (given only with the LayerNorm tail) is frozen."""
+
+    ARGS = ("x", "inp", "w_down", "b_down", "w_up", "b_up", "gamma", "beta", "eps", "act", "cache_d", "cache_u", "p", "F")
 
     @staticmethod
-    def forward(ctx, h, inp, w_down, b_down, w_up, b_up, gamma, beta, eps, act, cache_d, cache_u):
+    def forward(ctx, x, inp, w_down, b_down, w_up, b_up, gamma, beta, eps, act, cache_d, cache_u, p, F):
+        tail = 0 if gamma is not None else (1 if inp is not None else 2)
+        assert F is None or tail == 0, "a frozen F is fused only with the LayerNorm tail"
+        need = any(_needs(ctx, AdapterBlockFunction.ARGS).values())
+        h, u, rng = x, None, None
+        if F is not None:
+            rng = _dropout_rng(p, x, F)
+            h, u = _frozen_fwd(x, F, None, rng, need)
         wd, _ = cache_d.get(w_down)
         wu, _ = cache_u.get(w_up)
-        tail = 0 if gamma is not None else (1 if inp is not None else 2)
-        need = any(ctx.needs_input_grad[:8])
         g = b = None
         if tail == 0:
             g, b = gamma.detach().float().contiguous(), beta.detach().float().contiguous()
-        out, z, mean, rstd, s, u = ops.adapter_ln_fwd(h, inp, wd, b_down.detach().float().contiguous(), wu,
-                                                      b_up.detach().float().contiguous(), g, b, eps, act=act, tail=tail,
-                                                      save=need)
-        ctx.act, ctx.tail, ctx.caches, ctx.has_inp = act, tail, (cache_d, cache_u), inp is not None
-        if need:
-            ctx.save_for_backward(h, z, mean, rstd, g, s, u, w_down, w_up)
-        return out
-
-    @staticmethod
-    def backward(ctx, dout):
-        h, z, mean, rstd, g, s, u, w_down, w_up = ctx.saved_tensors
-        dout = dout.contiguous()
-        dg = db = None
-        if ctx.tail == 0:
-            if ctx.needs_input_grad[6] or ctx.needs_input_grad[7]:
-                dg, db = torch.empty_like(g), torch.empty_like(g)
-            dz = ops.layernorm_bwd(dout, z, mean, rstd, g, dgamma=dg, dbeta=db)
-        else:
-            dz = dout
-        _, wut = ctx.caches[1].get(w_up, need_t=True)      # [r, H]
-        _, wdt = ctx.caches[0].get(w_down, need_t=True)    # [H, r]
-        if ctx.act == "gelu":
-            ds = ops.gemm(dz, wut, epilogue=ops.EPI_DGELU, aux=u)
-        else:
-            ds = ops.gemm(dz, wut, epilogue=ops.EPI_DRELU, aux=s)
-        dh = ops.gemm(ds, wdt, residual=dz) if ctx.needs_input_grad[0] else None
-        dwd = ops.wgrad(ds, h) if ctx.needs_input_grad[2] else None
-        dbd = ops.colsum(ds) if ctx.needs_input_grad[3] else None
-        dwu = dbu = None
-        if ctx.needs_input_grad[4] or ctx.needs_input_grad[5]:
-            full = ops.wgrad(dz, ops.s_ext(s))               # dzᵀ · [s | 1]: weight and bias gradient in one pass over dz
-            dwu, dbu = full[:, :s.shape[1]], full[:, s.shape[1]]
-        dinp = dz if (ctx.has_inp and ctx.needs_input_grad[1]) else None
-        return dh, dinp, dwd, dbd, dwu, dbu, dg, db, None, None, None, None
-
-
-def houlsby_block(h, inp, adapter_down, adapter_up, act, ln=None):
-    """adapter_down / adapter_up: the AdapterBlock's Linear modules (weight, bias, _cache); ln: a LayerNorm module or None."""
-    return HoulsbyBlockFunction.apply(h, inp, adapter_down.weight, adapter_down.bias, adapter_up.weight, adapter_up.bias,
-                                      None if ln is None else ln.weight, None if ln is None else ln.bias,
-                                      0.0 if ln is None else ln.eps, act, adapter_down._cache, adapter_up._cache)
-
-
-class HoulsbyPostLNBlockFunction(torch.autograd.Function):
-    """One frozen post-LN block of BERT under a serial Houlsby wrapper (BertAdaptedSelfOutput.forward,
-    Downstream/Text/model/model.py:292-297) as a single autograd node:
-
-        h   = dropout(F(x))          F(x) = x Woᵀ + bo  (attention.output)  |  GELU(x Wiᵀ + bi) Wfᵀ + bf  (intermediate + output)
-        out = LayerNorm(h + W_u act(W_d h + b_d) + b_u + inp)
-
-    Forward: the dropout lives in the epilogue of F's last GEMM (counter RNG), everything after it is the fused K5 kernel.
-    Backward: LayerNorm backward -> two skinny data-gradient GEMMs; the second one forms (ds W_d + dz) and masks the SUM
-    with the regenerated dropout mask in its epilogue (`dropout_after_residual`), so no stand-alone dropout pass exists in
-    either direction; GELU' and — when `inp` is the block input x itself (the feed-forward block) — the skip gradient
-    ride in the epilogues of F's data-gradient GEMMs.  Trainable: the adapter and (finetune_layernorm) the LayerNorm."""
-
-    @staticmethod
-    def forward(ctx, x, inp, p, w1, b1, cache1, w2, b2, cache2, w_down, b_down, w_up, b_up, gamma, beta, eps, act,
-                cache_d, cache_u):
-        ffn = w2 is not None
-        need = ctx.needs_input_grad[0] or ctx.needs_input_grad[1] or any(ctx.needs_input_grad[9:15])
-        wa, _ = cache1.get(w1)
-        n_out = (w2 if ffn else w1).shape[0]
-        rng = (float(p),) + DropoutState.draw((x.shape[0] * n_out + 3) // 4) if p > 0 else None
-        u = None
-        if ffn:
-            wb, _ = cache2.get(w2)
-            u = torch.empty((x.shape[0], wa.shape[0]), dtype=BF16, device=x.device) if need else None
-            f = ops.gemm(x, wa, bias=b1.detach(), epilogue=ops.EPI_GELU, aux=u)
-            h = ops.gemm(f, wb, bias=b2.detach(), dropout=rng)
-        else:
-            h = ops.gemm(x, wa, bias=b1.detach(), dropout=rng)
-        wd, _ = cache_d.get(w_down)
-        wu, _ = cache_u.get(w_up)
-        g, b = gamma.detach().float().contiguous(), beta.detach().float().contiguous()
         out, z, mean, rstd, s, u_ad = ops.adapter_ln_fwd(h, inp, wd, b_down.detach().float().contiguous(), wu,
-                                                         b_up.detach().float().contiguous(), g, b, eps, act=act, tail=0,
+                                                         b_up.detach().float().contiguous(), g, b, eps, act=act, tail=tail,
                                                          save=need)
-        ctx.rng, ctx.ffn, ctx.act = rng, ffn, act
-        ctx.caches = (cache1, cache2, cache_d, cache_u)
-        ctx.inp_is_x = inp is x
-        if need:
-            ctx.save_for_backward(h, z, mean, rstd, g, s, u_ad, u, w1, w2, w_down, w_up)
+        ctx.act, ctx.tail, ctx.rng, ctx.F, ctx.caches = act, tail, rng, F, (cache_d, cache_u)
+        ctx.fold = F is not None and inp is x
+        ctx.save_for_backward(h, z, mean, rstd, g, s, u_ad, u, w_down, w_up)
         return out
 
     @staticmethod
     def backward(ctx, dout):
-        h, z, mean, rstd, g, s, u_ad, u, w1, w2, w_down, w_up = ctx.saved_tensors
-        cache1, cache2, cache_d, cache_u = ctx.caches
-        dout = dout.contiguous()
-        dg = db = None
-        if ctx.needs_input_grad[13] or ctx.needs_input_grad[14]:
-            dg, db = torch.empty_like(g), torch.empty_like(g)
-        dz = ops.layernorm_bwd(dout, z, mean, rstd, g, dgamma=dg, dbeta=db)
+        h, z, mean, rstd, g, s, u_ad, u, w_down, w_up = ctx.saved_tensors
+        need = _needs(ctx, AdapterBlockFunction.ARGS)
+        grads = {}
+        dz = dout.contiguous()
+        if ctx.tail == 0:
+            if need["gamma"] or need["beta"]:
+                grads["gamma"], grads["beta"] = torch.empty_like(g), torch.empty_like(g)
+            dz = ops.layernorm_bwd(dz, z, mean, rstd, g, dgamma=grads.get("gamma"), dbeta=grads.get("beta"))
+        cache_d, cache_u = ctx.caches
         _, wut = cache_u.get(w_up, need_t=True)      # [r, H]
         _, wdt = cache_d.get(w_down, need_t=True)    # [H, r]
         if ctx.act == "gelu":
             ds = ops.gemm(dz, wut, epilogue=ops.EPI_DGELU, aux=u_ad)
         else:
             ds = ops.gemm(dz, wut, epilogue=ops.EPI_DRELU, aux=s)
-        dwd = ops.wgrad(ds, h) if ctx.needs_input_grad[9] else None
-        dbd = ops.colsum(ds) if ctx.needs_input_grad[10] else None
-        dwu = dbu = None
-        if ctx.needs_input_grad[11] or ctx.needs_input_grad[12]:
+        if need["w_down"]:
+            grads["w_down"] = ops.wgrad(ds, h)
+        if need["b_down"]:
+            grads["b_down"] = ops.colsum(ds)
+        if need["w_up"] or need["b_up"]:
             full = ops.wgrad(dz, ops.s_ext(s))               # dzᵀ · [s | 1]: weight and bias gradient in one pass over dz
-            dwu, dbu = full[:, :s.shape[1]], full[:, s.shape[1]]
-        dx = None
-        if ctx.needs_input_grad[0]:
-            # gradient at the dense output, through the dropout: (ds W_d + dz) * mask / (1 - p) in ONE epilogue
-            dhm = ops.gemm(ds, wdt, residual=dz, dropout=ctx.rng, dropout_after=True)
-            fold = dz if ctx.inp_is_x else None
-            _, w1t = cache1.get(w1, need_t=True)
-            if ctx.ffn:
-                _, w2t = cache2.get(w2, need_t=True)
-                du = ops.gemm(dhm, w2t, epilogue=ops.EPI_DGELU, aux=u)
-                dx = ops.gemm(du, w1t, residual=fold)
-            else:
-                dx = ops.gemm(dhm, w1t, residual=fold)
-        dinp = dz if (ctx.needs_input_grad[1] and not ctx.inp_is_x) else None
-        return (dx, dinp, None, None, None, None, None, None, None, dwd, dbd, dwu, dbu, dg, db, None, None, None, None)
+            grads["w_up"], grads["b_up"] = full[:, :s.shape[1]], full[:, s.shape[1]]
+        if need["x"]:
+            # gradient at h, through F's dropout when there is one: (ds W_d + dz) * mask / (1 - p) in ONE epilogue
+            dh = ops.gemm(ds, wdt, residual=dz, dropout=ctx.rng, dropout_after=True)
+            grads["x"] = dh if ctx.F is None else _frozen_bwd(dh, u, ctx.F, dz if ctx.fold else None)
+        if need["inp"] and not ctx.fold:
+            grads["inp"] = dz
+        return tuple(grads.get(n) for n in AdapterBlockFunction.ARGS)
 
 
-def houlsby_postln_block(x, inp, p, dense, intermediate, adapter, ln):
-    """dense / intermediate: the frozen Linear modules of the block (intermediate None for attention.output);
-    adapter: the AdapterBlock; ln: the block's LayerNorm module."""
-    if intermediate is None:
-        w1, b1, c1, w2, b2, c2 = dense.weight, dense.bias, dense._cache, None, None, None
-    else:
-        w1, b1, c1 = intermediate.weight, intermediate.bias, intermediate._cache
-        w2, b2, c2 = dense.weight, dense.bias, dense._cache
-    return HoulsbyPostLNBlockFunction.apply(x, inp, p, w1, b1, c1, w2, b2, c2, adapter.fc_down.weight, adapter.fc_down.bias,
-                                            adapter.fc_up.weight, adapter.fc_up.bias, ln.weight, ln.bias, ln.eps,
-                                            adapter.act, adapter.fc_down._cache, adapter.fc_up._cache)
+def adapter_block(x, inp, adapter, ln=None, dense=None, intermediate=None, p=0.0):
+    """AdapterBlockFunction.  adapter: the AdapterBlock (fc_down, fc_up, act); ln: a LayerNorm module or None;
+    dense / intermediate: the frozen Linear modules of F (dense None: no F; intermediate None: F is dense alone)."""
+    d, up = adapter.fc_down, adapter.fc_up
+    return AdapterBlockFunction.apply(x, inp, d.weight, d.bias, up.weight, up.bias, *_ln_args(ln), adapter.act, d._cache,
+                                      up._cache, p, None if dense is None else _frozen(dense, intermediate))
 
 
 class IdEmbeddingFunction(torch.autograd.Function):

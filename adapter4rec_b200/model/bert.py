@@ -11,7 +11,7 @@ import torch.nn as nn
 
 from .. import functional as Fn
 from .. import ops
-from .layers import BF16, Embedding, LayerNorm, Linear, LoRALinear, to_2d_bf16
+from .layers import BF16, Embedding, LayerNorm, Linear, LoRALinear, frozen_ffn_dense, to_2d_bf16
 
 
 class TextConfigLite:
@@ -125,9 +125,7 @@ class BertSelfOutput(nn.Module):
         d = self.dense
         if not (d.weight.requires_grad or d.bias.requires_grad):
             # frozen dense: dense -> dropout -> + input -> LayerNorm as ONE autograd node (fused epilogues both ways)
-            out = Fn.PostLNBlockFunction.apply(to_2d_bf16(hidden_states), to_2d_bf16(input_tensor), self.LayerNorm.weight,
-                                               self.LayerNorm.bias, self.LayerNorm.eps, p, d.weight, d.bias, d._cache,
-                                               None, None, None)
+            out = Fn.frozen_block(to_2d_bf16(hidden_states), to_2d_bf16(input_tensor), d, ln=self.LayerNorm, p=p)
             return out.view(shape)
         if p > 0:
             z = Fn.dropout_add(d(to_2d_bf16(hidden_states)), to_2d_bf16(input_tensor).contiguous(), p)
@@ -183,24 +181,20 @@ class BertLayer(nn.Module):
             y = self.attention(x2d, attention_mask, N, L, packed)
         out = self.output
         wi = self.intermediate.dense
-        inner = out.self_output if hasattr(out, "self_output") else out          # Houlsby wrapper keeps the dense inside
-        wf = getattr(inner, "dense", None)
-        frozen = wf is not None and not (wi.weight.requires_grad or wi.bias.requires_grad or
-                                         wf.weight.requires_grad or wf.bias.requires_grad)
-        if frozen and type(out) is BertOutput:
+        wf = frozen_ffn_dense(wi, out)
+        if wf is not None and type(out) is BertOutput:
             # frozen feed-forward + dropout + residual + LayerNorm: one autograd node (GELU', dropout and the residual
             # gradient all live in GEMM / LayerNorm-backward epilogues)
             p = out.dropout.p if self.training else 0.0
-            return Fn.PostLNBlockFunction.apply(y, y, out.LayerNorm.weight, out.LayerNorm.bias, out.LayerNorm.eps, p,
-                                                wi.weight, wi.bias, wi._cache, wf.weight, wf.bias, wf._cache)
-        if frozen and hasattr(out, "forward_block"):
+            return Fn.frozen_block(y, y, wf, intermediate=wi, ln=out.LayerNorm, p=p)
+        if wf is not None and hasattr(out, "forward_block"):
             # serial Houlsby wrapper: FFN pair + dropout + adapter + LayerNorm in one autograd node
             fused = out.forward_block(y, y, wi)
             if fused is not None:
                 return to_2d_bf16(fused)
-        if frozen and hasattr(out, "forward_from_dense"):
+        if wf is not None and hasattr(out, "forward_from_dense"):
             # adapter-wrapped output: the frozen FFN pair stays fused, the wrapper continues from the dense output
-            h = Fn.FFNFunction.apply(y, wi.weight, wi.bias, wf.weight, wf.bias, None, wi._cache, wf._cache)
+            h = Fn.frozen_block(y, None, wf, intermediate=wi)
             return to_2d_bf16(out.forward_from_dense(h, y))
         return out(self.intermediate(y), y)                 # foreign or trainable output module
 

@@ -15,6 +15,16 @@ def to_2d_bf16(x):
     return x2 if x2.dtype == BF16 else x2.to(BF16)
 
 
+def frozen_ffn_dense(intermediate, output):
+    """The output dense Linear of a transformer layer's feed-forward pair (intermediate -> GELU -> output.dense) when
+    both Linears are frozen, else None.  `output` may be an adapter wrapper that keeps the original module as
+    `self_output`."""
+    dense = getattr(getattr(output, "self_output", output), "dense", None)
+    if dense is None or any(t.requires_grad for t in (intermediate.weight, intermediate.bias, dense.weight, dense.bias)):
+        return None
+    return dense
+
+
 class Linear(nn.Module):
     """nn.Linear replacement: parameters `weight` [out,in], `bias` [out] (fp32 masters), tcgen05 GEMM forward."""
 

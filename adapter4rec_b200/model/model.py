@@ -119,7 +119,7 @@ class BertAdaptedSelfOutput(nn.Module):
 
     def forward_block(self, x2, input_tensor, intermediate):
         """dense (or intermediate -> GELU -> dense when `intermediate` is given) -> dropout -> adapter -> LayerNorm as ONE
-        autograd node (Fn.HoulsbyPostLNBlockFunction) when the block's dense layers are frozen and the adapter has the
+        autograd node (Fn.AdapterBlockFunction) when the block's dense layers are frozen and the adapter has the
         fused kernel's shape; None otherwise (the caller composes the pieces)."""
         d = self.self_output.dense
         inp = x2 if input_tensor is x2 else to_2d_bf16(input_tensor)   # identity matters: inp is x folds the skip gradient
@@ -134,7 +134,8 @@ class BertAdaptedSelfOutput(nn.Module):
                 and inp.is_contiguous() and x2.shape[0] == inp.shape[0]):
             return None
         p = self.self_output.dropout.p if self.training else 0.0
-        out = Fn.houlsby_postln_block(x2, inp, p, d, intermediate, self.adapter, self.self_output.LayerNorm)
+        out = Fn.adapter_block(x2, inp, self.adapter, ln=self.self_output.LayerNorm, dense=d, intermediate=intermediate,
+                               p=p)
         return out.view(input_tensor.shape)
 
     def forward_from_dense(self, h, input_tensor):

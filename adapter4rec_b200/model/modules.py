@@ -189,7 +189,7 @@ class AdapterBlock(nn.Module):
 
     def fused(self, x2, extra_residual=None, ln=None):
         """tail(x + fc_up(act(fc_down(x))) [+ extra_residual]) in one kernel; tail = ln (a LayerNorm module) or identity"""
-        return Fn.houlsby_block(x2, extra_residual, self.fc_down, self.fc_up, self.act, ln=ln)
+        return Fn.adapter_block(x2, extra_residual, self, ln=ln)
 
 
 class AdapterPfeifferBlock(nn.Module):

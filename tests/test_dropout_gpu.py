@@ -157,9 +157,9 @@ def test_gemm_epilogue_dropout_before_and_after_the_residual(after, block_n, M, 
 
 
 def test_fused_houlsby_block_matches_the_composed_path_in_train_mode():
-    """HoulsbyPostLNBlockFunction (dense + dropout + adapter + LayerNorm in one node, dropout in GEMM epilogues both ways)
-    against dense -> a4r_dropout -> fused adapter block: both draw the same counters in the same order, so under one
-    seed the masks are identical and the results differ by bf16 rounding only."""
+    """AdapterBlockFunction with the frozen dense or FFN pair as F (F + dropout + adapter + LayerNorm in one node, dropout
+    in GEMM epilogues both ways) against F -> a4r_dropout -> the same node without F: both draw the same counters in the
+    same order, so under one seed the masks are identical and the results differ by bf16 rounding only."""
     import cases
     from adapter4rec_b200 import functional as Fn
     from adapter4rec_b200.model import model as M

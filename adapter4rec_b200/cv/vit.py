@@ -132,13 +132,11 @@ class ViTSelfAttention(nn.Module):
         self.query = Linear(config.hidden_size, config.hidden_size)
         self.key = Linear(config.hidden_size, config.hidden_size)
         self.value = Linear(config.hidden_size, config.hidden_size)
-        self._qkv_cache = {}
+        self._qkv_cache = Fn.QKVCache()
 
     def forward(self, x2d, N, L):
-        params = []
-        for m in (self.query, self.key, self.value):     # query / value may be loralib Linears (run_adapter.py:383-388)
-            params += [m.weight, m.bias, getattr(m, "lora_A", None), getattr(m, "lora_B", None)]
-        qkv = Fn.QKVFunction.apply(x2d, self._qkv_cache, *params)
+        # query / value may be loralib Linears (run_adapter.py:383-388)
+        qkv = Fn.qkv(x2d, (self.query, self.key, self.value), self._qkv_cache)
         return Fn.attention(qkv, None, N, L, self.num_attention_heads, self.attention_head_size, causal=False)
 
 

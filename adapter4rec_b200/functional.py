@@ -19,6 +19,13 @@ def bump_param_epoch():
     PARAM_EPOCH[0] += 1
 
 
+def _param_key(tensors):
+    """Staleness key of operands derived from `tensors` (None entries allowed): each tensor's storage and version, and
+    the optimizer-step count when any of them trains.  Operands are rebuilt when it changes."""
+    return tuple(None if t is None else (t.data_ptr(), t._version, t.device) for t in tensors) + (
+        PARAM_EPOCH[0] if any(t is not None and t.requires_grad for t in tensors) else -1,)
+
+
 class WeightCache:
     """bf16 copies of an fp32 master weight: W [N,K] for the forward GEMM and Wᵀ [K,N] for the data-gradient GEMM.
     Rebuilt when the parameter is modified in place (optimizer step, load_state_dict) or moved."""
@@ -30,7 +37,7 @@ class WeightCache:
         self.wt = None
 
     def get(self, weight, need_t=False):
-        key = (weight.data_ptr(), weight._version, weight.device, PARAM_EPOCH[0] if weight.requires_grad else -1)
+        key = _param_key((weight,))
         if key != self.key:
             self.key = key
             self.master = weight.detach()
@@ -239,7 +246,7 @@ def layer_norm(x, weight, bias, eps, res=None, res_param=None):
 class LayerNormSkipFunction(torch.autograd.Function):
     """(LN(x), x): a pre-LN block x1 = x + f(LN(x)) takes its skip connection from the SECOND output, so the skip gradient
     is delivered to this node and added inside the LayerNorm-backward kernel (a4r_layernorm_bwd_add) instead of by a
-    separate autograd accumulation pass over [M, H].  Same trick as QKVFunction's "skip" output on the post-LN side."""
+    separate autograd accumulation pass over [M, H].  Same trick as QKVFunction's skip output on the post-LN side."""
 
     @staticmethod
     def forward(ctx, x, weight, bias, eps):
@@ -442,176 +449,169 @@ def unique_rows(rows):
 LORA_PAD = 64  # the rank-r intermediates of all LoRA'd projections of one fused QKV share one 64-column k-block
 
 
+def _lora_slots(P):
+    """(slots, ones) of P = [(W, b, lora_A, lora_B) per projection]: slot (j, off, r) holds projection j's rank-r
+    intermediate in columns [off, off + r) of T; ones: the ranks leave column 63 of T free for a ones column"""
+    slots, off = [], 0
+    for j, (_, _, A, _) in enumerate(P):
+        if A is not None:
+            slots.append((j, off, A.shape[0]))
+            off += A.shape[0]
+    assert off <= LORA_PAD, "the LoRA ranks %s of one fused projection sum to %d, more than %d" % (
+        [r for _, _, r in slots], off, LORA_PAD)
+    return tuple(slots), bool(slots) and off < LORA_PAD
+
+
+class QKVCache:
+    """Operands of one QKVFunction: the bf16 fused weight [Wq;Wk;Wv], rebuilt when a weight changes (its transpose is
+    built by the first backward), and, rebuilt when any parameter changes, the fp32 fused bias (a missing bias is a block
+    of zeros) and the bf16 LoRA operands A_cat [64, K], A_catᵀ, B_ext [n·H, 64], B_extᵀ.  The LoRA tensors are written
+    into their slots of two persistent fp32 staging matrices (the padding stays zero) and the four operands come out of
+    two a4r_cast_transpose_f32_bf16 launches.  With a ones column, the constant bias of T = x·A_catᵀ sets column 63 to 1:
+    it adds nothing to qkv (B_ext[:, 63] = 0) and makes the bias gradients one more column of the dqkvᵀ·T gradient."""
+
+    def __init__(self):
+        self.w_key = self.key = self.layout = None
+        self.w = self.wt = self.bias = self.lora = None
+
+    def get(self, P, slots, ones):
+        """(W, bias, (T's bias, A_cat, A_catᵀ, B_ext, B_extᵀ) or None without LoRA)"""
+        key = _param_key([W for W, _, _, _ in P])
+        if key != self.w_key:
+            self.w_key, self.wt = key, None
+            self.w = torch.cat([W.detach().to(BF16) for W, _, _, _ in P], 0).contiguous()
+        key = _param_key([t for p in P for t in p])
+        if key != self.key:
+            self.key = key
+            self._build(P, slots, ones)
+        return self.w, self.bias, self.lora
+
+    def _build(self, P, slots, ones):
+        (H, K), dev = P[0][0].shape, P[0][0].device
+        layout = (dev, H, K, len(P), slots)
+        if layout != self.layout:
+            self.layout = layout
+            self.zero = torch.zeros(H, dtype=torch.float32, device=dev)
+            if slots:
+                self.stage = (torch.zeros((LORA_PAD, K), dtype=torch.float32, device=dev),
+                              torch.zeros((len(P) * H, LORA_PAD), dtype=torch.float32, device=dev))
+                self.t_bias = torch.zeros(LORA_PAD, dtype=torch.float32, device=dev)
+                if ones:
+                    self.t_bias[LORA_PAD - 1] = 1.0
+        self.bias = torch.cat([self.zero if b is None else b.detach().float() for _, b, _, _ in P])
+        self.lora = None
+        if slots:
+            a_stage, b_stage = self.stage
+            for j, o, r in slots:
+                a_stage[o:o + r].copy_(P[j][2].detach())
+                torch.mul(P[j][3].detach(), 1.0 / r, out=b_stage[j * H:(j + 1) * H, o:o + r])
+            self.lora = (self.t_bias,) + ops.cast_transpose(a_stage, True, True) + ops.cast_transpose(b_stage, True, True)
+
+    def weight_t(self):
+        if self.wt is None:
+            self.wt = self.w.t().contiguous()
+        return self.wt
+
+
 class QKVFunction(torch.autograd.Function):
     """Fused q|k|v projection of one attention module:  qkv = x·[Wq;Wk;Wv]ᵀ + [bq;bk;bv]  (one GEMM, N = 3H), where any
     of the three may be a loralib Linear (Downstream/Text/run.py:414-428):  + (x·Aᵀ)·Bᵀ / r.  The low-rank term rides in
     the same tcgen05 tile as a K-extension: T = x·A_catᵀ  [M,64]  is one skinny GEMM, then
     qkv = [x | T]·[W_cat | B_ext]ᵀ with B_ext the block matrix of the (scaled) lora_B factors.
 
-    params = (W, b, lora_A, lora_B) per fused projection (3 for q|k|v, 1 for a stand-alone loralib Linear), None where absent."""
+    params = (W, b, lora_A, lora_B) per fused projection (3 for q|k|v, 1 for a stand-alone loralib Linear), None where
+    absent; their operands come from `cache` (QKVCache).  with_skip: x is returned as a second output too.  A caller that
+    feeds it to the block's skip connection gets the skip gradient delivered to this node, where it rides in the epilogue
+    of the data-gradient GEMM instead of costing a separate elementwise add per layer."""
+
+    PARAMS = ("weight", "bias", "lora_A", "lora_B")
 
     @staticmethod
-    def forward(ctx, x, cache, *params):
-        """params may end with the marker string "skip": the function then ALSO returns x (as a second output).  A caller
-        that feeds this second output to the block's skip connection gets the skip gradient delivered to THIS node, where
-        it rides in the epilogue of the data-gradient GEMM instead of costing a separate elementwise add per layer."""
-        ctx.with_skip = len(params) > 0 and isinstance(params[-1], str) and params[-1] == "skip"
-        if ctx.with_skip:
-            params = params[:-1]
-        ctx.set_materialize_grads(False)
-        assert len(params) % 4 == 0
-        n = len(params) // 4
-        H = params[0].shape[0]
-        K = params[0].shape[1]
-        dev = x.device
-        frozen_w = not any(p is not None and p.requires_grad for p in [params[4 * j] for j in range(n)])
-        key = tuple((p.data_ptr(), p._version) for p in [params[4 * j] for j in range(n)]) + (PARAM_EPOCH[0] if not frozen_w else -1,)
-        if cache.get("key") != key or not frozen_w:
-            cache["key"] = key
-            cache["w"] = torch.cat([params[i].detach().to(BF16) for i in range(0, 4 * n, 4)], 0).contiguous()
-            cache["wt"] = None
-        w = cache["w"]
-        # the fused bias and the LoRA operand matrices depend on TRAINABLE tensors: rebuilt once per optimizer step (or
-        # whenever a parameter object / version changes), not once per forward
-        small = [params[4 * j + i] for j in range(n) for i in (1, 2, 3)]
-        skey = (PARAM_EPOCH[0],) + tuple(None if p is None else (p.data_ptr(), p._version) for p in small)
-        reuse = cache.get("small_key") == skey
-        if reuse:
-            bias = cache["bias"]
+    def args(n):
+        """argument names of the node over n projections; (j, name) is parameter `name` of projection j"""
+        return ("x", "cache", "with_skip") + tuple((j, p) for j in range(n) for p in QKVFunction.PARAMS)
+
+    @staticmethod
+    def forward(ctx, x, cache, with_skip, *params):
+        P = [params[i:i + 4] for i in range(0, len(params), 4)]
+        need = _needs(ctx, QKVFunction.args(len(P)))
+        slots, ones = _lora_slots(P)
+        w, bias, lora = cache.get(P, slots, ones)
+        T = a_cat_t = b_ext_t = None
+        if lora is None:
+            qkv = ops.gemm(x, w, bias=bias)
         else:
-            # one concatenation (a missing bias contributes a cached block of zeros)
-            zero_h = cache.get("zero_h")
-            if zero_h is None or zero_h.device != dev or zero_h.numel() != H:
-                zero_h = cache["zero_h"] = torch.zeros(H, dtype=torch.float32, device=dev)
-            bias = torch.cat([zero_h if params[4 * j + 1] is None else params[4 * j + 1].detach().float() for j in range(n)])
-            cache["small_key"], cache["bias"] = skey, bias
-        # LoRA bookkeeping: slot j occupies columns [off_j, off_j + r_j) of the 64-wide T
-        slots, off = [], 0
-        for j in range(n):
-            A = params[4 * j + 2]
-            if A is not None:
-                r = A.shape[0]
-                slots.append((j, off, r))
-                off += r
-        assert off <= LORA_PAD, "sum of LoRA ranks of one fused projection must be <= 64"
-        T = a_cat = b_ext = None
-        if slots:
-            ctx.ones_col = off < LORA_PAD
-            if reuse and "a_cat" in cache:
-                a_cat, b_ext, t_bias = cache["a_cat"], cache["b_ext"], cache["t_bias"]
-            else:
-                # Rebuilt once per optimizer step: the operands are assembled in two persistent fp32 staging matrices (the
-                # LoRA tensors are written straight into their slots, the padding stays zero) and every bf16 operand of the step
-                # — A_cat, A_catᵀ, B_ext, B_extᵀ — comes out of two a4r_cast_transpose_f32_bf16 launches.
-                st = cache.get("lora_stage")
-                if st is None or st[0].device != dev or st[0].shape != (LORA_PAD, K) or st[1].shape != (n * H, LORA_PAD):
-                    st = cache["lora_stage"] = (torch.zeros((LORA_PAD, K), dtype=torch.float32, device=dev),
-                                                torch.zeros((n * H, LORA_PAD), dtype=torch.float32, device=dev))
-                    cache["lora_slots"] = None
-                if cache.get("lora_slots") != slots:               # a different slot layout: clear what the old one wrote
-                    st[0].zero_()
-                    st[1].zero_()
-                    cache["lora_slots"] = list(slots)
-                for j, o, r in slots:
-                    st[0][o:o + r].copy_(params[4 * j + 2].detach())
-                    torch.mul(params[4 * j + 3].detach(), 1.0 / r, out=st[1][j * H:(j + 1) * H, o:o + r])
-                a_cat, a_cat_t = ops.cast_transpose(st[0], True, True)
-                b_ext, b_ext_t = ops.cast_transpose(st[1], True, True)
-                # column 63 of T is a constant 1 (zero weight row + bias 1): it contributes nothing to qkv (B_ext[:, 63] = 0)
-                # and turns the bias gradients into one more column of the fused dqkvᵀ·T weight-gradient below
-                tb = cache.get("t_bias_const")                      # (ones_col, tensor): a constant, built once
-                if tb is None or tb[0] != ctx.ones_col or tb[1].device != dev:
-                    t_bias = torch.zeros(LORA_PAD, dtype=torch.float32, device=dev)
-                    if ctx.ones_col:
-                        t_bias[LORA_PAD - 1] = 1.0
-                    tb = cache["t_bias_const"] = (ctx.ones_col, t_bias)
-                t_bias = tb[1]
-                cache["a_cat"], cache["b_ext"], cache["t_bias"] = a_cat, b_ext, t_bias
-                cache["a_cat_t"], cache["b_ext_t"] = a_cat_t, b_ext_t
+            t_bias, a_cat, a_cat_t, b_ext, b_ext_t = lora
             T = ops.gemm(x, a_cat, bias=t_bias)
             qkv = ops.gemm(x, w, bias=bias, a2=T, b2=b_ext)
-        else:
-            qkv = ops.gemm(x, w, bias=bias)
-        ctx.cache, ctx.slots, ctx.H, ctx.n = cache, slots, H, n
-        if not slots:
-            ctx.ones_col = False
-        ctx.n_params = len(params)
-        ctx.param_needs = [p is not None and p.requires_grad for p in params]
-        need_x = any(ctx.param_needs[4 * j + 2] for j in range(n)) or any(ctx.param_needs[4 * j] for j in range(n))
-        ctx.save_for_backward(x if need_x else None, T, a_cat, b_ext)
-        if ctx.with_skip:
-            return qkv, x          # autograd treats a returned input as x.view_as(x)
-        return qkv
+        ctx.set_materialize_grads(False)
+        ctx.cache, ctx.slots, ctx.ones, ctx.n, ctx.H = cache, slots, ones, len(P), P[0][0].shape[0]
+        need_x = any(need[(j, "weight")] or need[(j, "lora_A")] for j in range(len(P)))
+        ctx.save_for_backward(x if need_x else None, T, a_cat_t, b_ext_t)
+        return (qkv, x) if with_skip else qkv          # autograd treats a returned input as x.view_as(x)
 
     @staticmethod
     def backward(ctx, dqkv, dskip=None):
-        x, T, a_cat, b_ext = ctx.saved_tensors
-        H, cache, n = ctx.H, ctx.cache, ctx.n
-        tail = (None,) if ctx.with_skip else ()
+        x, T, a_cat_t, b_ext_t = ctx.saved_tensors
+        names = QKVFunction.args(ctx.n)
         if dqkv is None:                                  # only the skip output was used downstream
-            return (dskip, None) + (None,) * ctx.n_params + tail
-        dqkv = dqkv.contiguous()
-        if dskip is not None:
-            dskip = dskip.contiguous()
-        if cache.get("wt") is None:
-            cache["wt"] = cache["w"].t().contiguous()
-        grads = [None] * ctx.n_params
+            return (dskip,) + (None,) * (len(names) - 1)
+        need, grads = _needs(ctx, names), {}
+        H, n, slots = ctx.H, ctx.n, ctx.slots
+        third = lambda t, j: t[:, j * H:(j + 1) * H]
+        dqkv, dskip = dqkv.contiguous(), None if dskip is None else dskip.contiguous()
+        wt = ctx.cache.weight_t()
         dT = None
-        if ctx.slots:
-            # dT = dqkv·B_ext  [M,64];  dx = [dqkv | dT]·[W_catᵀ | A_catᵀ]ᵀ (+ the skip gradient in the epilogue)
-            if cache.get("b_ext") is b_ext and cache.get("b_ext_t") is not None:
-                b_ext_t, a_cat_t = cache["b_ext_t"], cache["a_cat_t"]
-            else:
-                b_ext_t, a_cat_t = b_ext.t().contiguous(), a_cat.t().contiguous()
-                if cache.get("b_ext") is b_ext:
-                    cache["b_ext_t"], cache["a_cat_t"] = b_ext_t, a_cat_t
-            # only the projections that carry a LoRA pair have non-zero rows in B_ext: with q|k|v fused and LoRA on q and v
-            # (run.py:414-428) the key third of dqkv is skipped — its products are exact zeros — so this HBM-bound skinny
-            # GEMM reads 2/3 of dqkv (two K-segments through the GEMM's second operand pair)
-            lj = [j for j, _, _ in ctx.slots]
-            if n == 3 and len(lj) == 2:
-                (ja, jb) = lj
-                dT = ops.gemm(dqkv[:, ja * H:(ja + 1) * H], b_ext_t[:, ja * H:(ja + 1) * H],
-                              a2=dqkv[:, jb * H:(jb + 1) * H], b2=b_ext_t[:, jb * H:(jb + 1) * H])
-            elif n == 3 and len(lj) == 1:
-                dT = ops.gemm(dqkv[:, lj[0] * H:(lj[0] + 1) * H], b_ext_t[:, lj[0] * H:(lj[0] + 1) * H])
-            else:
-                dT = ops.gemm(dqkv, b_ext_t)
-            dx = ops.gemm(dqkv, cache["wt"], a2=dT, b2=a_cat_t, residual=dskip) if ctx.needs_input_grad[0] else None
-        else:
-            dx = ops.gemm(dqkv, cache["wt"], residual=dskip) if ctx.needs_input_grad[0] else None
-        fused = bool(ctx.slots) and ctx.ones_col
-        if fused:
-            # ONE pass over dqkv gives every lora_B and every bias gradient; ONE pass over x gives every lora_A.  Each pass
-            # runs only if one of its results is wanted (x is saved only when a lora_A or a weight trains).
-            want_g1 = any(ctx.param_needs[4 * j + 1] for j in range(n)) or any(ctx.param_needs[4 * j + 3] for j, _, _ in ctx.slots)
-            want_g2 = any(ctx.param_needs[4 * j + 2] for j, _, _ in ctx.slots)
-            # g1 rows of projection j are wanted for its bias or its lora_B; a projection that needs neither (the frozen key
-            # projection under LoRA on q and v) is not read: one weight-gradient launch per wanted third of dqkv
-            g1_rows = [ctx.param_needs[4 * j + 1] or any(jj == j and ctx.param_needs[4 * j + 3] for jj, _, _ in ctx.slots)
-                       for j in range(n)]
+        if slots:
+            # dT = dqkv·B_ext [M,64].  B_ext has non-zero rows only in the thirds whose projection carries a LoRA pair, so
+            # this HBM-bound skinny GEMM reads those thirds of dqkv (one K-segment, or two through the second operand
+            # pair: LoRA on q and v, run.py:414-428, skips the key third), or all of dqkv when every projection has one
+            segs = [(dqkv, b_ext_t)] if len(slots) == n else [(third(dqkv, j), third(b_ext_t, j)) for j, _, _ in slots]
+            a2, b2 = segs[1] if len(segs) == 2 else (None, None)
+            dT = ops.gemm(*segs[0], a2=a2, b2=b2)
+        if need["x"]:                                     # dx = [dqkv | dT]·[W_cat ; A_cat] (+ the skip gradient)
+            grads["x"] = ops.gemm(dqkv, wt, a2=dT, b2=a_cat_t, residual=dskip)
+        if ctx.ones:
+            # ONE weight-gradient pass over a third of dqkv (over all of it when every third is wanted) gives that
+            # projection's bias and lora_B gradients, dqkvᵀ·[T | 1]; ONE pass over x gives every lora_A, dTᵀ·x (dT carries
+            # the 1/r of B_ext).  A third whose bias and lora_B need no gradient (the frozen key) is not read.
+            rows = [need[(j, "bias")] or need[(j, "lora_B")] for j in range(n)]
             g1 = [None] * n
-            if want_g1:
-                if all(g1_rows):
-                    full = ops.wgrad(dqkv, T)                       # [n*H, 64] = dqkvᵀ · [T | 1]
-                    g1 = [full[j * H:(j + 1) * H] for j in range(n)]
-                else:
-                    g1 = [ops.wgrad(dqkv[:, j * H:(j + 1) * H], T) if g1_rows[j] else None for j in range(n)]
-            g2 = ops.wgrad(dT, x) if want_g2 else None              # [64, K]   = dTᵀ · x
+            if all(rows):
+                full = ops.wgrad(dqkv, T)                                    # [n·H, 64]
+                g1 = [full[j * H:(j + 1) * H] for j in range(n)]
+            elif any(rows):
+                g1 = [ops.wgrad(third(dqkv, j), T) if rows[j] else None for j in range(n)]
+            g2 = ops.wgrad(dT, x) if any(need[(j, "lora_A")] for j in range(n)) else None      # [64, K]
+            bias_grad = lambda j: g1[j][:, LORA_PAD - 1].contiguous()
+            b_grad = lambda j, o, r: g1[j][:, o:o + r] * (1.0 / r)
+            a_grad = lambda o, r: g2[o:o + r].contiguous()
+        else:
+            # no LoRA, or ranks that fill all 64 columns of T: column sums, and weight gradients over aligned windows
+            bias_grad = lambda j: ops.colsum(third(dqkv, j))
+            b_grad = lambda j, o, r: _pad_cols_wgrad(third(dqkv, j), T, o, r, 1.0 / r, transpose=False)
+            a_grad = lambda o, r: _pad_cols_wgrad(dT, x, o, r, 1.0, transpose=True)
         for j in range(n):
-            dq = dqkv[:, j * H:(j + 1) * H]
-            if ctx.param_needs[4 * j]:
-                grads[4 * j] = ops.wgrad(dq, x)
-            if ctx.param_needs[4 * j + 1]:
-                grads[4 * j + 1] = g1[j][:, LORA_PAD - 1].contiguous() if fused else ops.colsum(dq)
-        for j, o, r in ctx.slots:
-            dq = dqkv[:, j * H:(j + 1) * H]
-            if ctx.param_needs[4 * j + 3]:   # lora_B [H, r] = (1/r) dqᵀ · T_j
-                grads[4 * j + 3] = (g1[j][:, o:o + r] * (1.0 / r)) if fused else \
-                    _pad_cols_wgrad(dq, T, o, r, 1.0 / r, transpose=False)
-            if ctx.param_needs[4 * j + 2]:   # lora_A [r, K] = dT_jᵀ · x   (dT already carries the 1/r of B_ext)
-                grads[4 * j + 2] = g2[o:o + r].contiguous() if fused else _pad_cols_wgrad(dT, x, o, r, 1.0, transpose=True)
-        return (dx, None) + tuple(grads) + tail
+            if need[(j, "weight")]:
+                grads[(j, "weight")] = ops.wgrad(third(dqkv, j), x)
+            if need[(j, "bias")]:
+                grads[(j, "bias")] = bias_grad(j)
+        for j, o, r in slots:
+            if need[(j, "lora_B")]:                      # lora_B [H, r] = (1/r) dq_jᵀ·T_j
+                grads[(j, "lora_B")] = b_grad(j, o, r)
+            if need[(j, "lora_A")]:                      # lora_A [r, K] = dT_jᵀ·x
+                grads[(j, "lora_A")] = a_grad(o, r)
+        return tuple(grads.get(k) for k in names)
+
+
+def qkv(x, modules, cache, skip=False):
+    """QKVFunction over the projection modules (query, key, value; any may be a LoRALinear) or one stand-alone
+    LoRALinear, with their QKVCache.  skip: returns (qkv, x') where x' is x as the node's second output (x itself when x
+    needs no gradient); the caller uses x' as the block's skip input."""
+    params = [getattr(m, name, None) for m in modules for name in QKVFunction.PARAMS]
+    with_skip = skip and x.requires_grad
+    out = QKVFunction.apply(x, cache, with_skip, *params)
+    return (out, x) if skip and not with_skip else out
 
 
 def _pad_cols_wgrad(a, b, off, r, alpha, transpose):

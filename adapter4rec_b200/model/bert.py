@@ -85,21 +85,16 @@ class BertSelfAttention(nn.Module):
         self.key = Linear(config.hidden_size, config.hidden_size)
         self.value = Linear(config.hidden_size, config.hidden_size)
         self.dropout = nn.Dropout(config.attention_probs_dropout_prob)
-        self._qkv_cache = {}
+        self._qkv_cache = Fn.QKVCache()
 
     def forward(self, x2d, attention_mask, N, L, packed=None, want_skip=False):
         """x2d bf16 [N*L, H]; attention_mask int64/f32 [N, L] (non-zero = attend) or None -> context [N*L, H].
         packed = PackedTokens: x2d holds only the kept tokens [T, H]; the mask is per token row.
         want_skip: also return x2d as an output of the projection's autograd node — the caller uses THAT tensor as the
         sub-layer's skip input, so the skip gradient is added inside the data-gradient GEMM's epilogue."""
-        params = []
-        for m in (self.query, self.key, self.value):     # any of them may have been replaced by a loralib Linear
-            params += [m.weight, m.bias, getattr(m, "lora_A", None), getattr(m, "lora_B", None)]
-        skip = x2d
-        if want_skip and x2d.requires_grad:
-            qkv, skip = Fn.QKVFunction.apply(x2d, self._qkv_cache, *params, "skip")
-        else:
-            qkv = Fn.QKVFunction.apply(x2d, self._qkv_cache, *params)
+        # any of query / key / value may have been replaced by a loralib Linear
+        out = Fn.qkv(x2d, (self.query, self.key, self.value), self._qkv_cache, skip=want_skip)
+        qkv, skip = out if want_skip else (out, None)
         if packed is not None:
             ctx = Fn.attention(qkv, packed.token_mask, N, L, self.num_attention_heads, self.attention_head_size,
                                causal=False, mask_neg=ops.F32_MIN, dropout_p=self.dropout.p if self.training else 0.0,

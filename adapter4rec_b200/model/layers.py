@@ -67,7 +67,7 @@ class LoRALinear(Linear):
             self.weight.requires_grad = False
             nn.init.kaiming_uniform_(self.lora_A, a=math.sqrt(5))
             nn.init.zeros_(self.lora_B)
-        self._qkv_cache = {}
+        self._qkv_cache = Fn.QKVCache()
 
     def forward(self, x, act=None, residual=None, residual2=None):
         if self.r == 0:
@@ -76,7 +76,7 @@ class LoRALinear(Linear):
         assert self.lora_alpha == 1, "only the reference's lora_alpha = 1 is implemented"
         shape = x.shape
         # stand-alone use: run the fused-projection function with a single slot
-        y = Fn.QKVFunction.apply(to_2d_bf16(x), self._qkv_cache, self.weight, self.bias, self.lora_A, self.lora_B)
+        y = Fn.qkv(to_2d_bf16(x), (self,), self._qkv_cache)
         return y.view(*shape[:-1], self.out_features)
 
 

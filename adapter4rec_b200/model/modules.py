@@ -65,15 +65,12 @@ class MultiHeadedAttention(nn.Module):
         self.self_attention = SelfAttention(temperature=self.d_k ** 0.5, dropout=dropout)
         self.dropout = nn.Dropout(p=dropout)
         self.layer_norm = LayerNorm(d_model, eps=1e-6)
-        self._qkv_cache = {}
+        self._qkv_cache = Fn.QKVCache()
 
     def presum(self, x2, mask, B, S, adapter=None, extra=None):
         """x2 + dropout(fc(attention(x2))) (+ extra) — the argument of the block's LayerNorm (see
         PositionwiseFeedForward.presum for `adapter` / `extra`)."""
-        params = []
-        for m in (self.w_Q, self.w_K, self.w_V):
-            params += [m.weight, m.bias, getattr(m, "lora_A", None), getattr(m, "lora_B", None)]
-        qkv = Fn.QKVFunction.apply(x2, self._qkv_cache, *params)
+        qkv = Fn.qkv(x2, (self.w_Q, self.w_K, self.w_V), self._qkv_cache)
         pd = self.self_attention.dropout.p if self.training else 0.0
         w = self.kernel_width(self.d_k)
         if w == self.d_k:
